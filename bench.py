@@ -3,7 +3,7 @@
 PointPillars front end -> BaseBEVBackbone -> shrink -> MessageExtractorv2 -> GenComm 3-step diffusion sampler ->
 Enhancer -> warp + AttFusion -> heads -> decode + rotated NMS), one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--shape opv2v_h|v2xreal]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--shape opv2v_h|v2xreal] [--dump-outputs DIR]
 
 A "step" is one pass of the whole frame path over F synthetic frames per GPU (F x 4 agents x 100 k points; --shape v2xreal:
 configs[3], 5 agents, C = 256).  Frames are independent, so ranks shard them (weak scaling); the path's one exchange step
@@ -297,8 +297,8 @@ class CpuFrame:
         return dt, (0 if boxes is None else int(boxes.shape[0]))
 
     def timed_frames(self, warmup, frames, seed0, budget_s):
-        """warmup untimed frames, then up to `frames` timed ones (stops early once budget_s of timed work is spent).
-        Returns (per-frame seconds, {stage: {median_ms, p90_ms}})."""
+        """warmup untimed frames, then up to `frames` timed ones (stops early once budget_s of timed work is spent, unless
+        budget_s is None).  Returns (per-frame seconds, {stage: {median_ms, p90_ms}})."""
         for w in range(warmup):
             self.run(10_000 + seed0 + w)
         tot, ts, per = 0.0, [], []
@@ -307,7 +307,7 @@ class CpuFrame:
             ts.append(dt)
             per.append(dict(self._cur))
             tot += dt
-            if tot > budget_s:
+            if budget_s is not None and tot > budget_s:
                 break
         stages = {}
         for name in list(_CPU_STAGES):
@@ -338,7 +338,7 @@ def run_reference(args):
     model, cores = cpu_info()
     torch.set_num_threads(cores)
     cpu = CpuFrame(shape)
-    ts, stages = cpu.timed_frames(max(args.warmup, 1), args.steps, 0, budget_s=120.0)
+    ts, stages = cpu.timed_frames(max(args.warmup, 1), args.steps, 0, budget_s=None)
     done, total = len(ts), float(np.sum(ts))
     fps = done / total
     k1 = None
@@ -364,7 +364,7 @@ def run_reference(args):
                                  "CPU voxelizer + H2D of the voxels + host NMS included as in the reference's loop"}
         except Exception as exc:
             gpu_eager = {"error": repr(exc)}
-    sample = (f"{done} frames timed after {max(args.warmup, 1)} warm-up (K = {args.steps} requested, 120 s cap), 1 frame per "
+    sample = (f"{done} frames timed after {max(args.warmup, 1)} warm-up, 1 frame per "
               f"step ({SHAPES[shape]['agents']} agents x 100k pts), torch CPU threads={cores}, {model}")
     print(json.dumps({
         "impl": "reference", "metric": SHAPES[shape]["metric"], "value": fps, "unit": "frames/s", "n_gpus": args.gpus,
@@ -515,6 +515,9 @@ def run_ours(args):
     rank, world, local = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
+    # the sampler noise is drawn on the device from the default CUDA generator, whose seed torch otherwise picks anew in
+    # every process: seeded, so that every run with the same arguments draws the same noise and finds the same boxes
+    torch.manual_seed(0)
     affinity = bind_to_gpu_numa(local)      # before any pinned allocation
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
@@ -609,7 +612,10 @@ def run_ours(args):
         barrier()
         elapsed_ms = t_start.elapsed_time(t_end)
     det_counts = (res[:, 0] if world > 1 else res[2].float()).tolist()
-    checksum = float((res if world > 1 else shard.pack_detections(*res)).double().sum().item())
+    payload = res if world > 1 else shard.pack_detections(*res)
+    checksum = float(payload.double().sum().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, payload)
 
     # ---------------- end-to-end timing: pinned host points -> device -> detections back in pinned host memory ----------------
     s_in, s_out = torch.cuda.Stream(), torch.cuda.Stream()
@@ -779,6 +785,30 @@ STAGE_KERNELS = {
 }
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, payload):
+    """--dump-outputs: the detections of the last timed step, i.e. what the callers of DetectorPipeline.step receive
+    (every rank's frames when N > 1), as out_dir/{frames,counts,scores,boxes}.npy: frame indices (float64), then float32
+    counts [n], scores [n,1000] and boxes [n,1000,8,3] with the rows beyond each frame's count zeroed (gc_postprocess
+    leaves them unspecified).  The inputs, and the sampler noise drawn from the seeded CUDA generator in a fixed order,
+    are the same from run to run for the same arguments, so two builds can be compared output for output.  Above 64 MB
+    a fixed, seeded sample of the frames is written."""
+    p = payload.cpu().numpy()
+    n, top = p.shape[0], (p.shape[1] - 1) // 25      # a row: count | scores [top] | boxes [top, 8, 3]
+    frames = np.arange(n)
+    keep = DUMP_LIMIT_BYTES // (p.shape[1] * 4 + 8)
+    if n > keep:
+        frames = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        p = p[frames]
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"frames": frames.astype(np.float64), "counts": p[:, 0], "scores": p[:, 1:1 + top],
+              "boxes": p[:, 1 + top:].reshape(len(frames), top, 8, 3)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
 def pipeline_launches(pipe, stage_ms):
     """Kernels of this repo launched per detector step (counted from the launch sequence of each stage; the torch.randn /
     elementwise launches of the wrappers are not counted)."""
@@ -867,7 +897,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary sections (configs[1] HBM step, sampler, ...)")
     ap.add_argument("--cpu-protocol", action="store_true", help="--impl reference: also time k = 1 thread (BASELINE.md section 3)")
     ap.add_argument("--no-gpu-eager", action="store_true", help="--impl reference: skip the torch-eager-on-GPU bar")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the detections of the last timed step as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     # The contract is ONE JSON line on stdout.  Libraries write to fd 1 behind Python's back (NCCL prints its version
     # banner there at communicator creation), so fd 1 is pointed at stderr for the whole run and the JSON line goes to a
     # private duplicate of the original stdout.
