@@ -36,10 +36,12 @@ def test_det_tail_matches_golden(golden_det_tail):
         _close(r.cpu(), T(g[f"head{i}/out"]), f"head{i}")
 
 
-@pytest.mark.parametrize("cin,cout,H,W,stride,N", [(384, 128, 128, 256, 2, 1), (256, 128, 64, 128, 1, 2), (64, 256, 8, 48, 1, 1)])
+@pytest.mark.parametrize("cin,cout,H,W,stride,N", [(384, 128, 128, 256, 2, 1), (256, 128, 64, 128, 1, 2), (64, 256, 8, 48, 1, 1),
+                                                   (384, 256, 128, 256, 2, 8)])
 def test_downsample_conv_matches_oracle(cin, cout, H, W, stride, N):
-    """The GenComm stage-1 shrink header (384 -> 128, stride 2, 128x256 -> 64x128), a stride-1 header, and a 256-column
-    case with rows that are not a multiple of the tile."""
+    """The GenComm stage-1 shrink header (384 -> 128, stride 2, 128x256 -> 64x128), a stride-1 header, a 256-column
+    case with rows that are not a multiple of the tile, and the configs[3] header (384 -> 256) over 8 agents: 512 tiles,
+    three or more per CTA pair of the multicast kernel."""
     torch.manual_seed(cin + H)
     cfg = {"kernal_size": [3], "stride": [stride], "padding": [1], "dim": [cout], "input_dim": cin}
     m = DownsampleConv(cfg).eval()
@@ -50,13 +52,15 @@ def test_downsample_conv_matches_oracle(cin, cout, H, W, stride, N):
 
 
 def test_det_heads_match_oracle_and_errors():
-    torch.manual_seed(2)
-    heads = DetectionHeads(128, 2).eval()
-    x = synth.bev_features(66, 3, 128, 64, 128)
-    ref = R.det_heads(x, *[t.detach() for h in (heads.cls_head, heads.reg_head, heads.dir_head) for t in (h.weight, h.bias)])
-    got = heads.to(DEV)(x.to(DEV))
-    for name, a, b in zip(("cls", "reg", "dir"), got, ref):
-        _close(a.cpu(), b, name)
+    """C = 128 (OPV2V-H) over 3 frames and C = 256 (V2X-Real) over 8 frames (512 tiles: three or more per CTA)."""
+    for C, B in ((128, 3), (256, 8)):
+        torch.manual_seed(2)
+        heads = DetectionHeads(C, 2).eval()
+        x = synth.bev_features(66, B, C, 64, 128)
+        ref = R.det_heads(x, *[t.detach() for h in (heads.cls_head, heads.reg_head, heads.dir_head) for t in (h.weight, h.bias)])
+        got = heads.to(DEV)(x.to(DEV))
+        for name, a, b in zip(("cls", "reg", "dir"), got, ref):
+            _close(a.cpu(), b, f"{name} C={C}")
     with pytest.raises(RuntimeError, match="multiple of 128"):
         heads(torch.zeros(1, 128, 3, 10, device=DEV))
     bad = DownsampleConv({"kernal_size": [3], "stride": [1], "padding": [1], "dim": [64], "input_dim": 48}).to(DEV)

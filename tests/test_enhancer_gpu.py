@@ -30,10 +30,11 @@ def test_enhancer_matches_golden(golden_enhancer):
     _close(out, T(g["ref_out"]), "enhancer")
 
 
-@pytest.mark.parametrize("C,H,W,N", [(128, 64, 128, 2), (256, 8, 48, 2), (128, 2, 64, 1)])
+@pytest.mark.parametrize("C,H,W,N", [(128, 64, 128, 2), (256, 8, 48, 2), (128, 2, 64, 1), (256, 64, 128, 8)])
 def test_enhancer_matches_oracle(C, H, W, N):
-    """OPV2V-H (C=128, 64x128) and V2X-Real (C=256) shapes, rows that are not a multiple of the 128-pixel tile, against
-    the oracle restatement on the same seeded inputs and randomised LayerNorm / bias parameters."""
+    """OPV2V-H (C=128, 64x128) and V2X-Real (C=256) shapes, rows that are not a multiple of the 128-pixel tile, and
+    C=256 at 64x128 over 8 agents (the GEMMs on CTA pairs, three or more tiles per CTA), against the oracle restatement on
+    the same seeded inputs and randomised LayerNorm / bias parameters."""
     torch.manual_seed(C + W)
     model = Enhancer(C, [8, 8], 4).eval()
     with torch.no_grad():

@@ -57,9 +57,10 @@ def test_message_extractor_matches_golden(golden_message_extractor):
     assert torch.equal(out2, out)
 
 
-@pytest.mark.parametrize("C,H,W,N,scale", [(128, 64, 128, 2, 4.0), (256, 8, 48, 1, 1.0), (64, 2, 64, 3, 8.0), (64, 3, 256, 2, 2.0)])
+@pytest.mark.parametrize("C,H,W,N,scale", [(128, 64, 128, 2, 4.0), (256, 8, 48, 1, 1.0), (64, 2, 64, 3, 8.0), (64, 3, 256, 2, 2.0),
+                                                    (256, 64, 128, 5, 4.0)])
 def test_message_extractor_matches_oracle(C, H, W, N, scale):
-    """OPV2V-H (C=128, 64x128) and V2X-Real-like (C=256) shapes, rows that are not a multiple of the 128-pixel tile
+    """OPV2V-H (C=128, 64x128) and V2X-Real-like (C=256, also at 64x128 over 5 agents) shapes, rows that are not a multiple of the 128-pixel tile
     (W=48), rows of two tiles (W=256: the row-staged offset fast path with interior tile edges), large offsets (taps
     leave the image) -- against the oracle restatement on the same seeded inputs."""
     torch.manual_seed(C + H)
