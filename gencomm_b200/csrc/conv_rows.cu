@@ -238,8 +238,7 @@ k_conv_rows(const uint4 *__restrict__ xh, const uint4 *__restrict__ xl, const ui
 }
 
 template <int NOUT, int R, int NB, int EPI>
-static int launch(cudaStream_t st, int A, const uint4 *xh, const uint4 *xl, const uint4 *wp, const float *bias, int C, int H, int W,
-                  int out_ch_total, int out_ch_off, float *out, uint4 *oh, uint4 *ol) {
+static int launch(cudaStream_t st, const ConvLayer &L) {
     constexpr int kSmem = smem_bytes(NOUT, R, NB);
     static_assert(kSmem <= 226 * 1024, "k_conv_rows: shared memory");
     static int sms = 0;
@@ -251,35 +250,30 @@ static int launch(cudaStream_t st, int A, const uint4 *xh, const uint4 *xl, cons
         if (e != cudaSuccess || n <= 0) { (void)cudaGetLastError(); set_error("k_conv_rows: launch set-up failed (%d)", (int)e); return e != cudaSuccess ? (int)e : (int)cudaErrorUnknown; }
         sms = n;
     }
-    const int n_tiles = A * (W / 128) * (H / R);
-    k_conv_rows<NOUT, R, NB, EPI><<<n_tiles < sms ? n_tiles : sms, kThreads, kSmem, st>>>(xh, xl, wp, bias, n_tiles, C, H, W, out_ch_total,
-                                                                                         out_ch_off, out, oh, ol);
+    const int H = L.Ho(), W = L.Wo(), n_tiles = L.A * (W / 128) * (H / R);
+    k_conv_rows<NOUT, R, NB, EPI><<<n_tiles < sms ? n_tiles : sms, kThreads, kSmem, st>>>(L.xh, L.xl, L.w, L.bias, n_tiles, L.c_in, H, W,
+                                                                                         L.out_ch_total, L.out_ch_off, L.out, L.oh, L.ol);
     GC_LAUNCH_CHECK("k_conv_rows");
     return GC_OK;
 }
 
 }  // namespace cr
 
-bool conv_rows_eligible(int taps, int stride, int c_in, int n_out, int H, int W) {
+bool conv_rows_eligible(const ConvLayer &L) {
     // opt-in since k_conv_tma: the TMA-fed kernel runs the same layers faster (32 agents: 64 ch 263 vs 276 us, 128 ch 166 vs 214 us).
     // Read per call so that a test can run both paths in one process.
     const char *e = getenv("GC_CONV_ROWS");
     if (!(e && e[0] == '1')) return false;
-    if (taps != 9 || stride != 1 || W % 128 != 0 || c_in % 32 != 0) return false;
-    if (n_out == 64) return H % 4 == 0;
-    if (n_out == 128) return H % 2 == 0;
+    if (L.taps != 9 || L.stride != 1 || L.up != 1 || (L.epi != 3 && L.epi != 5) || L.c_in != L.C || L.Wo() % 128 != 0 || L.c_in % 32 != 0)
+        return false;
+    if (L.n_out == 64) return L.Ho() % 4 == 0;
+    if (L.n_out == 128) return L.Ho() % 2 == 0;
     return false;
 }
 
-int conv_rows(cudaStream_t st, int A, const void *xh, const void *xl, const void *packed, const float *bias, int c_in, int n_out,
-              int H, int W, int out_ch_total, int out_ch_off, float *out_nchw, void *oh, void *ol) {
-    const uint4 *a = (const uint4 *)xh, *b = (const uint4 *)xl, *w = (const uint4 *)packed;
-    if (n_out == 64) {
-        if (oh) return cr::launch<64, 4, 3, 5>(st, A, a, b, w, bias, c_in, H, W, out_ch_total, out_ch_off, nullptr, (uint4 *)oh, (uint4 *)ol);
-        return cr::launch<64, 4, 3, 3>(st, A, a, b, w, bias, c_in, H, W, out_ch_total, out_ch_off, out_nchw, nullptr, nullptr);
-    }
-    if (oh) return cr::launch<128, 2, 4, 5>(st, A, a, b, w, bias, c_in, H, W, out_ch_total, out_ch_off, nullptr, (uint4 *)oh, (uint4 *)ol);
-    return cr::launch<128, 2, 4, 3>(st, A, a, b, w, bias, c_in, H, W, out_ch_total, out_ch_off, out_nchw, nullptr, nullptr);
+int conv_rows(cudaStream_t st, const ConvLayer &L) {
+    if (L.n_out == 64) return L.epi == 5 ? cr::launch<64, 4, 3, 5>(st, L) : cr::launch<64, 4, 3, 3>(st, L);
+    return L.epi == 5 ? cr::launch<128, 2, 4, 5>(st, L) : cr::launch<128, 2, 4, 3>(st, L);
 }
 
 }  // namespace gc

@@ -5,52 +5,18 @@
 //   models/sub_modules/downsample_conv.py:7-50   DoubleConv = Conv2d(k, stride s, pad) + ReLU + Conv2d(3x3, pad 1) + ReLU,
 //                                                DownsampleConv = a list of them (shipped configs: one 3x3 layer, stride 1 or 2)
 //   models/heter_model_baseline.py:130-135        cls_head / reg_head / dir_head: three 1x1 Conv2d on the fused feature
-// All of it runs through the tcgen05 implicit-GEMM kernel of implicit_gemm.cuh in bf16x3 (value + residual bf16 planes of
-// both operands, fp32 accumulation in TMEM: fp32-grade results): strided / plain 3x3 with a bias + ReLU epilogue, and
-// ONE 1x1 GEMM for the three heads (their weight matrices concatenated, N <= 64).
+// All of it runs as plane-convolution layers (conv_layer.cuh) in bf16x3 (value + residual bf16 planes of both operands, fp32
+// accumulation in TMEM: fp32-grade results): strided / plain 3x3 with a bias + ReLU epilogue, and ONE 1x1 GEMM for the three
+// heads (their weight matrices concatenated, N <= 64).
 #include "common.cuh"
-#include <stdlib.h>
 
-#include "conv_tma.cuh"
-#include "conv_rows.cuh"
-#include "implicit_gemm.cuh"
+#include "conv_layer.cuh"
 
 namespace gc {
 namespace dt {
 
-using namespace me;
-constexpr int kSc = 32;
-
-template <int NOUT, int TAPS, int EPI>
-static int launch(cudaStream_t st, dim3 grid, const uint4 *xh, const uint4 *xl, const uint4 *wp, const float *bias, int C, int H,
-                  int W, int n_store, float *out, int H_in, int W_in, int stride) {
-    if (ct::conv_tma_eligible(stride, C, C, H, W, 1))
-        return ct::launch_conv_tma<NOUT, TAPS, EPI>(st, (int)grid.y, xh, xl, wp, bias, C, C, H, W, H_in, W_in, stride, n_store, n_store, 0,
-                                                    out, nullptr, nullptr, 1, 0, 0);
-    constexpr int kSmem = conv_smem_bytes(NOUT, true, kSc);
-    static bool done = false;
-    if (!done) {
-        cudaFuncSetAttribute(k_me_conv<NOUT, false, kSc, TAPS, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
-        done = true;
-    }
-    k_me_conv<NOUT, false, kSc, TAPS, EPI><<<grid, conv_block_threads(false), kSmem, st>>>(xh, xl, nullptr, wp, bias, C, C, H, W, n_store,
-                                                                       n_store, 0, out, nullptr, H_in, W_in, stride);
-    GC_LAUNCH_CHECK("k_me_conv (det_tail)");
-    return GC_OK;
-}
-
-template <int TAPS, int EPI>
-static int launch_n(int n, cudaStream_t st, dim3 grid, const uint4 *xh, const uint4 *xl, const uint4 *wp, const float *bias,
-                    int C, int H, int W, float *out, int H_in, int W_in, int stride) {
-    if (n <= 32) return launch<32, TAPS, EPI>(st, grid, xh, xl, wp, bias, C, H, W, n, out, H_in, W_in, stride);
-    if (n <= 64) return launch<64, TAPS, EPI>(st, grid, xh, xl, wp, bias, C, H, W, n, out, H_in, W_in, stride);
-    if (n <= 128) return launch<128, TAPS, EPI>(st, grid, xh, xl, wp, bias, C, H, W, n, out, H_in, W_in, stride);
-    return launch<256, TAPS, EPI>(st, grid, xh, xl, wp, bias, C, H, W, n, out, H_in, W_in, stride);
-}
-static inline int pad_n(int n) { return n <= 32 ? 32 : n <= 64 ? 64 : n <= 128 ? 128 : 256; }
-static int double_conv_from_planes(cudaStream_t st, int A, const uint4 *xh, const uint4 *xl, int c_in, int H, int W, int stride,
-                                   int c_out, const void *packed, const float *bias, float *mid, float *out);
-static inline size_t packed_conv_bytes(int taps, int cin, int n) { return (size_t)taps * cin * pad_n(n) * 2 * 2; }
+// both convolutions of a DoubleConv are packed for N = conv_n_pad(c_out, 32), the second at a 256-byte boundary
+static inline size_t second_conv_off(int c_in, int c_out) { return align_up(conv_packed_bytes(9, c_in, conv_n_pad(c_out, 32)), 256); }
 
 struct Ws {
     uint4 *xh, *xl;   // channel-last planes of the current layer's input (sized for the larger of the two layers)
@@ -74,6 +40,22 @@ static Ws carve(void *base, int A, int cin, int hw_in, int n1, int hw_out) {
     return w;
 }
 
+// DoubleConv on channel-last planes: conv3x3(stride) + ReLU written as planes into `mid` (two planes of A*c_out*Ho*Wo*2 bytes
+// = the bytes of one fp32 tensor), conv3x3 + ReLU -> fp32 NCHW.  No fp32 intermediate, no second layout conversion.
+static int double_conv_from_planes(cudaStream_t st, int A, const uint4 *xh, const uint4 *xl, int c_in, int H, int W, int stride,
+                                   int c_out, const void *packed, const float *bias, float *mid, float *out) {
+    ConvLayer L;
+    L.xh = xh; L.xl = xl; L.A = A; L.C = L.c_in = c_in; L.H_in = H; L.W_in = W; L.taps = 9; L.stride = stride;
+    L.w = (const uint4 *)packed; L.n_pad = conv_n_pad(c_out, 32); L.bias = bias; L.n_out = L.out_ch_total = c_out;
+    L.epi = 5; L.oh = (uint4 *)mid; L.ol = (uint4 *)((char *)mid + (size_t)A * c_out * L.Ho() * L.Wo() * 2);
+    if (int rc = conv_layer(st, L)) return rc;
+    ConvLayer L2 = L;   // the second convolution: stride 1 over the planes the first wrote
+    L2.xh = L.oh; L2.xl = L.ol; L2.C = L2.c_in = c_out; L2.H_in = L.Ho(); L2.W_in = L.Wo(); L2.stride = 1;
+    L2.w = (const uint4 *)((const char *)packed + second_conv_off(c_in, c_out)); L2.bias = bias + c_out;
+    L2.epi = 3; L2.out = out; L2.oh = L2.ol = nullptr;
+    return conv_layer(st, L2);
+}
+
 }  // namespace dt
 }  // namespace gc
 
@@ -81,26 +63,19 @@ using namespace gc;
 
 extern "C" size_t gc_double_conv_packed_bytes(int c_in, int c_out) {
     if (c_in <= 0 || c_out <= 0) return 0;
-    return align_up(dt::packed_conv_bytes(9, c_in, c_out), 256) + dt::packed_conv_bytes(9, c_out, c_out);
+    return dt::second_conv_off(c_in, c_out) + conv_packed_bytes(9, c_out, conv_n_pad(c_out, 32));
 }
 extern "C" size_t gc_double_conv_workspace_bytes(int total_agents, int c_in, int H, int W, int stride, int c_out) {
     if (total_agents <= 0 || c_in <= 0 || c_out <= 0 || H <= 0 || W <= 0 || stride <= 0) return 0;
-    const int Ho = (H + 2 - 3) / stride + 1, Wo = (W + 2 - 3) / stride + 1;
-    return dt::carve(nullptr, total_agents, c_in, H * W, c_out, Ho * Wo).bytes;
+    return dt::carve(nullptr, total_agents, c_in, H * W, c_out, conv_out_size(H, stride) * conv_out_size(W, stride)).bytes;
 }
 extern "C" int gc_double_conv_pack(const float *w1, const float *w2, int c_in, int c_out, void *packed, void *stream) {
     GC_REQUIRE(w1 && w2 && packed, GC_EINVAL, "gc_double_conv_pack: null pointer");
     GC_REQUIRE(c_in > 0 && c_in % 64 == 0 && c_out > 0 && c_out % 64 == 0 && c_out <= 256, GC_EUNSUPPORTED,
                "gc_double_conv_pack: channels must be multiples of 64, c_out <= 256 (got %d -> %d)", c_in, c_out);
     cudaStream_t st = (cudaStream_t)stream;
-    const int n = dt::pad_n(c_out);
-    const int t1 = 9 * (c_in / 8) * n, t2 = 9 * (c_out / 8) * n;
-    me::k_me_pack<<<(t1 + 255) / 256, 256, 0, st>>>(w1, c_out, n, c_in, dt::kSc, 9, 1, (uint4 *)packed);
-    GC_LAUNCH_CHECK("k_me_pack(double_conv.0)");
-    me::k_me_pack<<<(t2 + 255) / 256, 256, 0, st>>>(
-        w2, c_out, n, c_out, dt::kSc, 9, 1, (uint4 *)((char *)packed + align_up(dt::packed_conv_bytes(9, c_in, c_out), 256)));
-    GC_LAUNCH_CHECK("k_me_pack(double_conv.2)");
-    return GC_OK;
+    if (int rc = conv_pack(st, w1, 9, c_in, c_out, 32, packed)) return rc;
+    return conv_pack(st, w2, 9, c_out, c_out, 32, (char *)packed + dt::second_conv_off(c_in, c_out));
 }
 
 extern "C" int gc_double_conv(const float *x, int total_agents, int c_in, int H, int W, int stride, int c_out,
@@ -112,23 +87,18 @@ extern "C" int gc_double_conv(const float *x, int total_agents, int c_in, int H,
     GC_REQUIRE(c_in > 0 && c_in % 64 == 0 && c_out > 0 && c_out % 64 == 0 && c_out <= 256, GC_EUNSUPPORTED,
                "gc_double_conv: channels must be multiples of 64, c_out <= 256 (got %d -> %d)", c_in, c_out);
     GC_REQUIRE(stride == 1 || stride == 2, GC_EUNSUPPORTED, "gc_double_conv: stride must be 1 or 2 (got %d)", stride);
-    const int Ho = (H + 2 - 3) / stride + 1, Wo = (W + 2 - 3) / stride + 1;
-    GC_REQUIRE(H > 0 && W > 0 && (Ho * Wo) % me::kPix == 0, GC_EUNSUPPORTED,
+    const int Ho = conv_out_size(H, stride), Wo = conv_out_size(W, stride);
+    GC_REQUIRE(H > 0 && W > 0 && (Ho * Wo) % 128 == 0, GC_EUNSUPPORTED,
                "gc_double_conv: output H*W must be a multiple of 128 (got %dx%d)", Ho, Wo);
     cudaStream_t st = (cudaStream_t)stream;
     const int A = total_agents;
     const dt::Ws ws = dt::carve(workspace, A, c_in, H * W, c_out, Ho * Wo);
-    const uint4 *p1 = (const uint4 *)packed;
-    const uint4 *p2 = (const uint4 *)((const char *)packed + align_up(dt::packed_conv_bytes(9, c_in, c_out), 256));
-    const dim3 grid(Ho * Wo / me::kPix, A);
-    me::k_me_to_nhwc<<<dim3((H * W + 63) / 64, c_in / 64, A), 256, 0, st>>>(x, c_in, H * W, ws.xh, ws.xl);
-    GC_LAUNCH_CHECK("k_me_to_nhwc(x)");
+    if (int rc = to_planes(st, x, A, c_in, H * W, ws.xh, ws.xl)) return rc;
     return dt::double_conv_from_planes(st, A, ws.xh, ws.xl, c_in, H, W, stride, c_out, packed, bias, ws.mid, out);
 }
 extern "C" size_t gc_double_conv_planes_workspace_bytes(int total_agents, int H, int W, int stride, int c_out) {
     if (total_agents <= 0 || c_out <= 0 || H <= 0 || W <= 0 || stride <= 0) return 0;
-    const int Ho = (H + 2 - 3) / stride + 1, Wo = (W + 2 - 3) / stride + 1;
-    return align_up((size_t)total_agents * c_out * Ho * Wo * 4, 256);
+    return align_up((size_t)total_agents * c_out * conv_out_size(H, stride) * conv_out_size(W, stride) * 4, 256);
 }
 extern "C" int gc_double_conv_planes(const void *xh, const void *xl, int total_agents, int c_in, int H, int W, int stride, int c_out,
                                      const void *packed, const float *bias /* [2][c_out] */, void *workspace, float *out,
@@ -139,14 +109,16 @@ extern "C" int gc_double_conv_planes(const void *xh, const void *xl, int total_a
     GC_REQUIRE(c_in > 0 && c_in % 64 == 0 && c_out > 0 && c_out % 64 == 0 && c_out <= 256, GC_EUNSUPPORTED,
                "gc_double_conv_planes: channels must be multiples of 64, c_out <= 256 (got %d -> %d)", c_in, c_out);
     GC_REQUIRE(stride == 1 || stride == 2, GC_EUNSUPPORTED, "gc_double_conv_planes: stride must be 1 or 2 (got %d)", stride);
-    const int Ho = (H + 2 - 3) / stride + 1, Wo = (W + 2 - 3) / stride + 1;
-    GC_REQUIRE(H > 0 && W > 0 && (Ho * Wo) % me::kPix == 0, GC_EUNSUPPORTED,
+    const int Ho = conv_out_size(H, stride), Wo = conv_out_size(W, stride);
+    GC_REQUIRE(H > 0 && W > 0 && (Ho * Wo) % 128 == 0, GC_EUNSUPPORTED,
                "gc_double_conv_planes: output H*W must be a multiple of 128 (got %dx%d)", Ho, Wo);
     return dt::double_conv_from_planes((cudaStream_t)stream, total_agents, (const uint4 *)xh, (const uint4 *)xl, c_in, H, W, stride,
                                        c_out, packed, bias, (float *)workspace, out);
 }
 
-extern "C" size_t gc_det_heads_packed_bytes(int C, int n_out) { return C > 0 && n_out > 0 ? dt::packed_conv_bytes(1, C, n_out) : 0; }
+extern "C" size_t gc_det_heads_packed_bytes(int C, int n_out) {
+    return C > 0 && n_out > 0 ? conv_packed_bytes(1, C, conv_n_pad(n_out, 32)) : 0;
+}
 extern "C" size_t gc_det_heads_workspace_bytes(int n_frames, int C, int H, int W) {
     if (n_frames <= 0 || C <= 0 || H <= 0 || W <= 0) return 0;
     return 2 * align_up((size_t)n_frames * H * W * C * 2, 256);
@@ -155,10 +127,7 @@ extern "C" int gc_det_heads_pack(const float *w /* [n_out][C] */, int C, int n_o
     GC_REQUIRE(w && packed, GC_EINVAL, "gc_det_heads_pack: null pointer");
     GC_REQUIRE(C > 0 && C % 64 == 0 && n_out > 0 && n_out <= 64, GC_EUNSUPPORTED,
                "gc_det_heads_pack: C must be a multiple of 64 and n_out <= 64 (got %d, %d)", C, n_out);
-    const int n = dt::pad_n(n_out), t = (C / 8) * n;
-    me::k_me_pack<<<(t + 255) / 256, 256, 0, (cudaStream_t)stream>>>(w, n_out, n, C, dt::kSc, 1, 1, (uint4 *)packed);
-    GC_LAUNCH_CHECK("k_me_pack(heads)");
-    return GC_OK;
+    return conv_pack((cudaStream_t)stream, w, 1, C, n_out, 32, packed);
 }
 extern "C" int gc_det_heads(const float *x, int n_frames, int C, int H, int W, int n_out, const void *packed,
                             const float *bias /* [n_out] */, void *workspace, float *out /* [B][n_out][H][W] */,
@@ -168,153 +137,15 @@ extern "C" int gc_det_heads(const float *x, int n_frames, int C, int H, int W, i
     GC_REQUIRE(x && packed && bias && workspace && out, GC_EINVAL, "gc_det_heads: null pointer");
     GC_REQUIRE(C > 0 && C % 64 == 0 && n_out > 0 && n_out <= 64, GC_EUNSUPPORTED,
                "gc_det_heads: C must be a multiple of 64 and n_out <= 64 (got %d, %d)", C, n_out);
-    GC_REQUIRE(H > 0 && W > 0 && (H * W) % me::kPix == 0, GC_EUNSUPPORTED,
+    GC_REQUIRE(H > 0 && W > 0 && (H * W) % 128 == 0, GC_EUNSUPPORTED,
                "gc_det_heads: H*W must be a multiple of 128 (got %dx%d)", H, W);
     cudaStream_t st = (cudaStream_t)stream;
-    uint4 *xh = (uint4 *)workspace;
-    uint4 *xl = (uint4 *)((char *)workspace + align_up((size_t)n_frames * H * W * C * 2, 256));
-    me::k_me_to_nhwc<<<dim3((H * W + 63) / 64, C / 64, n_frames), 256, 0, st>>>(x, C, H * W, xh, xl);
-    GC_LAUNCH_CHECK("k_me_to_nhwc(fused)");
-    return dt::launch_n<1, 0>(n_out, st, dim3(H * W / me::kPix, n_frames), xh, xl, (const uint4 *)packed, bias, C, H, W, out, H,
-                              W, 1);
-}
-
-// ------------------------------------------------------------------------------------------------
-// Generic layer entry points over the channel-last bf16 planes (used by the host mirror of BaseBEVBackbone,
-// models/sub_modules/base_bev_backbone.py:96-124): conv3x3 (stride 1/2, pad 1) or 1x1, folded-BN bias, ReLU, written
-// either as the next layer's planes or as NCHW fp32 (optionally pixel-shuffled = one phase of a ConvTranspose2d whose
-// kernel equals its stride).
-// ------------------------------------------------------------------------------------------------
-namespace gc {
-namespace dt {
-
-template <int NOUT, int TAPS, int EPI, int MT>
-static int launch_layer_mt(cudaStream_t st, dim3 grid, const uint4 *xh, const uint4 *xl, const uint4 *wp, const float *bias, int C,
-                           int Ho, int Wo, int n_out, int out_total, int out_off, float *out, uint4 *oh, uint4 *ol, int H_in,
-                           int W_in, int stride, int up, int up_dy, int up_dx) {
-    if (MT == 1 && ct::conv_tma_eligible(stride, C, C, Ho, Wo, up))
-        return ct::launch_conv_tma<NOUT, TAPS, EPI>(st, (int)grid.y, xh, xl, wp, bias, C, C, Ho, Wo, H_in, W_in, stride, n_out, out_total,
-                                                    out_off, out, oh, ol, up, up_dy, up_dx);
-    constexpr int kSmem = conv_smem_bytes(NOUT, true, kSc, MT);
-    static bool done = false;
-    if (!done) {
-        cudaFuncSetAttribute(k_me_conv<NOUT, false, kSc, TAPS, EPI, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
-        done = true;
-    }
-    grid.x /= MT;
-    k_me_conv<NOUT, false, kSc, TAPS, EPI, MT><<<grid, conv_block_threads(false), kSmem, st>>>(
-        xh, xl, nullptr, wp, bias, C, C, Ho, Wo, n_out, out_total, out_off, out, nullptr, H_in, W_in, stride, oh, ol, up, up_dy, up_dx);
-    GC_LAUNCH_CHECK("k_me_conv (layer)");
-    return GC_OK;
-}
-// 3x3 plane-to-plane layers (the backbone's bulk) can run two 128-pixel tiles per CTA on one weight stage (half the weight
-// traffic from L2).  Measured on the B200: backbone 7.89 ms vs 7.66 ms with one tile -- no gain, so it is opt-in.
-template <int NOUT, int TAPS, int EPI>
-static int launch_layer(cudaStream_t st, dim3 grid, const uint4 *xh, const uint4 *xl, const uint4 *wp, const float *bias, int C,
-                        int Ho, int Wo, int n_out, int out_total, int out_off, float *out, uint4 *oh, uint4 *ol, int H_in,
-                        int W_in, int stride, int up, int up_dy, int up_dx) {
-    static const bool two = getenv("GC_CONV_MT2") != nullptr;   // measured: no gain (DESIGN.md 5e), opt-in for A/B
-    if constexpr (TAPS == 9 && EPI == 5) {
-        if (two && grid.x % 2 == 0 && (long long)grid.x * grid.y >= 2 * 148)
-            return launch_layer_mt<NOUT, TAPS, EPI, 2>(st, grid, xh, xl, wp, bias, C, Ho, Wo, n_out, out_total, out_off, out, oh, ol,
-                                                       H_in, W_in, stride, up, up_dy, up_dx);
-    }
-    return launch_layer_mt<NOUT, TAPS, EPI, 1>(st, grid, xh, xl, wp, bias, C, Ho, Wo, n_out, out_total, out_off, out, oh, ol, H_in,
-                                               W_in, stride, up, up_dy, up_dx);
-}
-template <int TAPS, int EPI, class... Args>
-static int launch_layer_n(int n, Args... args) {
-    if (n <= 64) return launch_layer<64, TAPS, EPI>(args...);
-    if (n <= 128) return launch_layer<128, TAPS, EPI>(args...);
-    return launch_layer<256, TAPS, EPI>(args...);
-}
-
-// DoubleConv on channel-last planes: conv3x3(stride) + ReLU written as planes into `mid` (two planes of A*c_out*Ho*Wo*2 bytes
-// = the bytes of one fp32 tensor), conv3x3 + ReLU -> fp32 NCHW.  No fp32 intermediate, no second layout conversion.
-static int double_conv_from_planes(cudaStream_t st, int A, const uint4 *xh, const uint4 *xl, int c_in, int H, int W, int stride,
-                                   int c_out, const void *packed, const float *bias, float *mid, float *out) {
-    const int Ho = (H + 2 - 3) / stride + 1, Wo = (W + 2 - 3) / stride + 1;
-    const uint4 *p1 = (const uint4 *)packed;
-    const uint4 *p2 = (const uint4 *)((const char *)packed + align_up(packed_conv_bytes(9, c_in, c_out), 256));
-    const dim3 grid(Ho * Wo / me::kPix, A);
-    uint4 *mh = (uint4 *)mid, *ml = (uint4 *)((char *)mid + (size_t)A * c_out * Ho * Wo * 2);
-    if (stride == 1 && conv_rows_eligible(9, 1, c_in, c_out, Ho, Wo)) {
-        if (int rc = conv_rows(st, A, xh, xl, p1, bias, c_in, c_out, Ho, Wo, c_out, 0, nullptr, mh, ml)) return rc;
-    } else if (int rc = launch_layer_n<9, 5>(c_out, st, grid, xh, xl, p1, bias, c_in, Ho, Wo, c_out, c_out, 0, (float *)nullptr, mh, ml,
-                                             H, W, stride, 1, 0, 0)) {
-        return rc;
-    }
-    if (conv_rows_eligible(9, 1, c_out, c_out, Ho, Wo))
-        return conv_rows(st, A, mh, ml, p2, bias + c_out, c_out, c_out, Ho, Wo, c_out, 0, out, nullptr, nullptr);
-    return launch_layer_n<9, 3>(c_out, st, grid, (const uint4 *)mh, (const uint4 *)ml, p2, bias + c_out, c_out, Ho, Wo, c_out, c_out,
-                                0, out, (uint4 *)nullptr, (uint4 *)nullptr, Ho, Wo, 1, 1, 0, 0);
-}
-
-}  // namespace dt
-}  // namespace gc
-
-extern "C" size_t gc_conv_packed_bytes(int taps, int c_in, int n_out) {
-    return (taps == 1 || taps == 9) && c_in > 0 && n_out > 0 ? dt::packed_conv_bytes(taps, c_in, n_out < 64 ? 64 : n_out) : 0;
-}
-extern "C" int gc_conv_pack(const float *w /* [n_out][c_in][taps] */, int taps, int c_in, int n_out, void *packed, void *stream) {
-    GC_REQUIRE(w && packed, GC_EINVAL, "gc_conv_pack: null pointer");
-    GC_REQUIRE((taps == 1 || taps == 9) && c_in > 0 && c_in % 32 == 0 && n_out > 0 && n_out <= 256, GC_EUNSUPPORTED,
-               "gc_conv_pack: taps in {1,9}, c_in %% 32 == 0, n_out <= 256 (got %d, %d, %d)", taps, c_in, n_out);
-    const int n = dt::pad_n(n_out < 64 ? 64 : n_out), t = taps * (c_in / 8) * n;
-    me::k_me_pack<<<(t + 255) / 256, 256, 0, (cudaStream_t)stream>>>(w, n_out, n, c_in, dt::kSc, taps, 1, (uint4 *)packed);
-    GC_LAUNCH_CHECK("k_me_pack(layer)");
-    return GC_OK;
-}
-extern "C" int gc_to_planes(const float *x, int total_agents, int C, int HW, void *xh, void *xl, void *stream) {
-    GC_REQUIRE(total_agents >= 0 && C > 0 && C % 64 == 0 && HW > 0, GC_EUNSUPPORTED, "gc_to_planes: C must be a multiple of 64");
-    if (total_agents == 0) return GC_OK;
-    GC_REQUIRE(x && xh && xl, GC_EINVAL, "gc_to_planes: null pointer");
-    me::k_me_to_nhwc<<<dim3((HW + 63) / 64, C / 64, total_agents), 256, 0, (cudaStream_t)stream>>>(x, C, HW, (uint4 *)xh, (uint4 *)xl);
-    GC_LAUNCH_CHECK("k_me_to_nhwc");
-    return GC_OK;
-}
-extern "C" int gc_conv_planes(const void *xh, const void *xl, int total_agents, int c_in, int H_in, int W_in, int stride, int taps,
-                              int n_out, const void *packed, const float *bias, void *oh, void *ol, float *out_nchw,
-                              int out_ch_total, int out_ch_off, int up, int up_dy, int up_dx, void *stream) {
-    GC_REQUIRE(total_agents >= 0 && total_agents <= 65535, GC_EINVAL, "gc_conv_planes: bad agent count");
-    if (total_agents == 0) return GC_OK;
-    GC_REQUIRE(xh && xl && packed && ((oh && ol) || out_nchw), GC_EINVAL, "gc_conv_planes: null pointer");
-    GC_REQUIRE((taps == 1 || taps == 9) && c_in > 0 && c_in % 32 == 0 && n_out >= 8 && n_out <= 256 && n_out % 8 == 0,
-               GC_EUNSUPPORTED, "gc_conv_planes: taps in {1,9}, c_in %% 32 == 0, n_out %% 8 == 0, n_out <= 256");
-    GC_REQUIRE((stride == 1 || stride == 2) && (taps == 9 || stride == 1) && up >= 1 &&
-                   ((up_dy >= 0 && up_dy < up && up_dx >= 0 && up_dx < up) || (up_dy == -1 && taps == 1)),
-               GC_EUNSUPPORTED, "gc_conv_planes: bad stride / up-sampling phase");
-    if (up_dy == -1 && !(ct::conv_tma_eligible(stride, c_in, c_in, H_in, W_in, up) && n_out % 16 == 0 && n_out >= 64)) {
-        // all phases requested but the fused launch does not apply: one launch per phase
-        const size_t phase_bytes = gc_conv_packed_bytes(1, c_in, n_out);
-        for (int ph = 0; ph < up * up; ++ph)
-            if (int rc = gc_conv_planes(xh, xl, total_agents, c_in, H_in, W_in, stride, taps, n_out, (const char *)packed + ph * phase_bytes,
-                                        bias, oh, ol, out_nchw, out_ch_total, out_ch_off, up, ph / up, ph % up, stream))
-                return rc;
-        return GC_OK;
-    }
-    const int Ho = taps == 9 ? (H_in - 1) / stride + 1 : H_in, Wo = taps == 9 ? (W_in - 1) / stride + 1 : W_in;
-    GC_REQUIRE(Ho > 0 && Wo > 0 && (Ho * Wo) % me::kPix == 0, GC_EUNSUPPORTED,
-               "gc_conv_planes: output H*W must be a multiple of 128 (got %dx%d)", Ho, Wo);
-    GC_REQUIRE(out_ch_total >= out_ch_off + n_out && out_ch_total % 8 == 0 && out_ch_off % 8 == 0, GC_EINVAL,
-               "gc_conv_planes: bad output channel window");
-    cudaStream_t st = (cudaStream_t)stream;
-    const dim3 grid(Ho * Wo / me::kPix, total_agents);
-    const uint4 *a = (const uint4 *)xh, *b = (const uint4 *)xl, *wp = (const uint4 *)packed;
-    // wide stride-1 layers: the row-staged kernel (conv_rows.cu) reads every input row once per channel chunk instead of nine times
-    if (up == 1 && conv_rows_eligible(taps, stride, c_in, n_out, Ho, Wo))
-        return conv_rows(st, total_agents, xh, xl, packed, bias, c_in, n_out, Ho, Wo, out_ch_total, out_ch_off, out_nchw, oh, ol);
-    if (oh) {
-        GC_REQUIRE(n_out % 16 == 0, GC_EUNSUPPORTED, "gc_conv_planes: plane outputs need n_out %% 16 == 0");
-        if (taps == 9)
-            return dt::launch_layer_n<9, 5>(n_out, st, grid, a, b, wp, bias, c_in, Ho, Wo, n_out, out_ch_total, out_ch_off,
-                                            (float *)nullptr, (uint4 *)oh, (uint4 *)ol, H_in, W_in, stride, up, up_dy, up_dx);
-        return dt::launch_layer_n<1, 5>(n_out, st, grid, a, b, wp, bias, c_in, Ho, Wo, n_out, out_ch_total, out_ch_off,
-                                        (float *)nullptr, (uint4 *)oh, (uint4 *)ol, H_in, W_in, stride, up, up_dy, up_dx);
-    }
-    if (taps == 9)
-        return dt::launch_layer_n<9, 3>(n_out, st, grid, a, b, wp, bias, c_in, Ho, Wo, n_out, out_ch_total, out_ch_off, out_nchw,
-                                        (uint4 *)nullptr, (uint4 *)nullptr, H_in, W_in, stride, up, up_dy, up_dx);
-    return dt::launch_layer_n<1, 3>(n_out, st, grid, a, b, wp, bias, c_in, Ho, Wo, n_out, out_ch_total, out_ch_off, out_nchw,
-                                    (uint4 *)nullptr, (uint4 *)nullptr, H_in, W_in, stride, up, up_dy, up_dx);
+    ConvLayer L;
+    L.xh = (const uint4 *)workspace;
+    L.xl = (const uint4 *)((char *)workspace + align_up((size_t)n_frames * H * W * C * 2, 256));
+    if (int rc = to_planes(st, x, n_frames, C, H * W, (void *)L.xh, (void *)L.xl)) return rc;
+    L.A = n_frames; L.C = L.c_in = C; L.H_in = H; L.W_in = W; L.taps = 1;
+    L.w = (const uint4 *)packed; L.n_pad = conv_n_pad(n_out, 32); L.bias = bias; L.n_out = L.out_ch_total = n_out;
+    L.epi = 0; L.out = out;
+    return conv_layer(st, L);
 }

@@ -9,12 +9,12 @@
 //   :286-314  SplitAttn.forward        global average pool -> fc1 -> LayerNorm -> ReLU -> fc2 -> sigmoid -> scale
 // Everything is per agent, so all agents of all frames run in one pass (regroup / record_len only split and re-join).
 //
-// The three dense contractions (98 % of the 1.8 GFLOP per agent at C = 128) run on tcgen05 through the implicit-GEMM
-// kernel of implicit_gemm.cuh in "bf16x3" (value + residual bf16 planes of both operands, three MMAs per K = 16 step,
+// The three dense contractions (98 % of the 1.8 GFLOP per agent at C = 128) run on tcgen05 as plane-convolution layers
+// (conv_layer.cuh) in "bf16x3" (value + residual bf16 planes of both operands, three MMAs per K = 16 step,
 // fp32 accumulation in TMEM -- fp32-grade results):
-//   partial_conv3 : k_me_conv<C/4, plain 3x3>           K = 9 C/4
-//   linear1+GELU  : k_me_conv<256, 1x1, GELU> x C/64    K = C,   N = 4C in chunks of 256 TMEM columns
-//   linear2       : k_me_conv<128, 1x1>       x C/128   K = 2C,  N = C
+//   partial_conv3 : N = C/4, plain 3x3           K = 9 C/4
+//   linear1+GELU  : N = 256, 1x1, GELU  x C/64   K = C,   N = 4C in chunks of 256 TMEM columns
+//   linear2       : N = 128, 1x1        x C/128  K = 2C,  N = C
 // fed by k_me_to_nhwc (NCHW fp32 -> channel-last bf16 planes).  LayerNorms, the depth-wise convolution + gate, the
 // pool / excite and the final scale are fp32 CUDA-core kernels (thread = pixel, plane-coalesced).
 // linear1 writes its GELU'd output channel-last (fp32) and the depth-wise + gate kernel turns it directly into linear2's
@@ -22,7 +22,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
-#include "conv_tma.cuh"
+#include "conv_layer.cuh"
 #include "implicit_gemm.cuh"
 
 namespace gc {
@@ -261,32 +261,13 @@ static Workspace carve(void *base, int A, int C, int HW) {
     return w;
 }
 
-// packed bf16x3 B operands: [partial_conv3][linear1: C/32 chunks of 128 rows][linear2: C/128 chunks of 128 rows]
-constexpr int kSc = 32;
-static inline size_t pk_pconv_bytes(int C) { return (size_t)9 * (C / 4) * (C / 4) * 2 * 2; }      // N = C/4 rows
-static inline size_t pk_lin1_chunk_bytes(int C) { return (size_t)C * 256 * 2 * 2; }   // 256 rows per launch
-static inline size_t pk_lin2_chunk_bytes(int C) { return (size_t)2 * C * 128 * 2 * 2; }
+// packed bf16x3 B operands: [partial_conv3][linear1: C/64 chunks of 256 rows][linear2: C/128 chunks of 128 rows]
+static inline size_t pk_pconv_bytes(int C) { return conv_packed_bytes(9, C / 4, C / 4); }     // N = C/4 rows
+static inline size_t pk_lin1_chunk_bytes(int C) { return conv_packed_bytes(1, C, 256); }   // 256 rows per launch
+static inline size_t pk_lin2_chunk_bytes(int C) { return conv_packed_bytes(1, 2 * C, 128); }
 static inline size_t pk_lin1_off(int C) { return align_up(pk_pconv_bytes(C), 256); }
 static inline size_t pk_lin2_off(int C) { return pk_lin1_off(C) + (size_t)(C / 64) * pk_lin1_chunk_bytes(C); }
 static inline size_t pk_total(int C) { return pk_lin2_off(C) + (size_t)(C / 128) * pk_lin2_chunk_bytes(C); }
-
-template <int NOUT, int TAPS, int EPI>
-static int launch_conv(cudaStream_t st, dim3 grid, const uint4 *xh, const uint4 *xl, const uint4 *wp, const float *bias, int C,
-                       int c_in, int H, int W, int n_store, int out_total, int out_off, float *out) {
-    if (ct::conv_tma_eligible(1, C, c_in, H, W, 1))      // TMA-fed persistent kernel (conv_tma.cuh), bit-identical results
-        return ct::launch_conv_tma<NOUT, TAPS, EPI>(st, (int)grid.y, xh, xl, wp, bias, C, c_in, H, W, H, W, 1, n_store, out_total, out_off,
-                                                    out, nullptr, nullptr, 1, 0, 0);
-    constexpr int kSmem = conv_smem_bytes(NOUT, true, kSc);
-    static bool done = false;
-    if (!done) {
-        cudaFuncSetAttribute(k_me_conv<NOUT, false, kSc, TAPS, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
-        done = true;
-    }
-    k_me_conv<NOUT, false, kSc, TAPS, EPI><<<grid, conv_block_threads(false), kSmem, st>>>(xh, xl, nullptr, wp, bias, C, c_in, H, W, n_store,
-                                                                       out_total, out_off, out, nullptr);
-    GC_LAUNCH_CHECK("k_me_conv (enhancer)");
-    return GC_OK;
-}
 
 }  // namespace enh
 }  // namespace gc
@@ -307,24 +288,13 @@ extern "C" int gc_enhancer_pack_weights(const float *w_pconv, const float *w_lin
     cudaStream_t st = (cudaStream_t)stream;
     char *pk = (char *)packed;
     const int c4 = C / 4;
-    {   // partial_conv3.weight [C/4][C/4][3][3]
-        const int n = 9 * (c4 / 8) * c4;
-        me::k_me_pack<<<(n + 255) / 256, 256, 0, st>>>(w_pconv, c4, c4, c4, enh::kSc, 9, 1, (uint4 *)pk);
-        GC_LAUNCH_CHECK("k_me_pack(partial_conv3)");
-    }
-    for (int j = 0; j < C / 64; ++j) {   // linear1.weight [4C][C], rows 256 j ..
-        const int n = (C / 8) * 256;
-        me::k_me_pack<<<(n + 255) / 256, 256, 0, st>>>(w_lin1 + (size_t)j * 256 * C, 256, 256, C, enh::kSc, 1, 1,
-                                                      (uint4 *)(pk + enh::pk_lin1_off(C) + j * enh::pk_lin1_chunk_bytes(C)));
-        GC_LAUNCH_CHECK("k_me_pack(linear1)");
-    }
-    for (int j = 0; j < C / 128; ++j) {   // linear2.weight [C][2C], rows 128 j ..
-        const int n = (2 * C / 8) * 128;
-        me::k_me_pack<<<(n + 255) / 256, 256, 0, st>>>(w_lin2 + (size_t)j * 128 * 2 * C, 128, 128, 2 * C, enh::kSc, 1, 1,
-                                                      (uint4 *)(pk + enh::pk_lin2_off(C) + j * enh::pk_lin2_chunk_bytes(C)));
-        GC_LAUNCH_CHECK("k_me_pack(linear2)");
-    }
-    return GC_OK;
+    // partial_conv3.weight [C/4][C/4][3][3]
+    int rc = conv_pack(st, w_pconv, 9, c4, c4, 32, pk);
+    for (int j = 0; j < C / 64 && !rc; ++j)   // linear1.weight [4C][C], rows 256 j ..
+        rc = conv_pack(st, w_lin1 + (size_t)j * 256 * C, 1, C, 256, 32, pk + enh::pk_lin1_off(C) + j * enh::pk_lin1_chunk_bytes(C));
+    for (int j = 0; j < C / 128 && !rc; ++j)   // linear2.weight [C][2C], rows 128 j ..
+        rc = conv_pack(st, w_lin2 + (size_t)j * 128 * 2 * C, 1, 2 * C, 128, 32, pk + enh::pk_lin2_off(C) + j * enh::pk_lin2_chunk_bytes(C));
+    return rc;
 }
 
 extern "C" int gc_enhancer(const float *x, int total_agents, int C, int H, int W, const void *packed, const float *params,
@@ -345,33 +315,34 @@ extern "C" int gc_enhancer(const float *x, int total_agents, int C, int H, int W
 
     enh::k_enh_ln<<<grid, 128, 0, st>>>(x, params, L, C, HW, ws.x1, ws.y);
     GC_LAUNCH_CHECK("k_enh_ln");
-    me::k_me_to_nhwc<<<dim3((HW + 63) / 64, C / 64, A), 256, 0, st>>>(ws.y, C, HW, ws.yh, ws.yl);
-    GC_LAUNCH_CHECK("k_me_to_nhwc(y)");
+    if ((rc = to_planes(st, ws.y, A, C, HW, ws.yh, ws.yl))) return rc;
     // partial_conv3 on the first C/4 channels, written over planes 0 .. C/4-1 of y (it reads the bf16 planes, not y)
-    if (c4 == 32)
-        rc = enh::launch_conv<32, 9, 0>(st, grid, ws.yh, ws.yl, (const uint4 *)pk, nullptr, C, c4, H, W, c4, C, 0, ws.y);
-    else
-        rc = enh::launch_conv<64, 9, 0>(st, grid, ws.yh, ws.yl, (const uint4 *)pk, nullptr, C, c4, H, W, c4, C, 0, ws.y);
-    if (rc) return rc;
-    me::k_me_to_nhwc<<<dim3((HW + 63) / 64, C / 64, A), 256, 0, st>>>(ws.y, C, HW, ws.yh, ws.yl);
-    GC_LAUNCH_CHECK("k_me_to_nhwc(ycat)");
-    for (int j = 0; j < C / 64; ++j) {   // linear1 + GELU, 256 output channels (= 256 TMEM columns) per launch: the A
-        // operand is staged once per 256 columns (128 per launch was measured first: 4 x 125 us at C = 128)
-        rc = enh::launch_conv<256, 1, 2>(st, grid, ws.yh, ws.yl,
-                                         (const uint4 *)(pk + enh::pk_lin1_off(C) + j * enh::pk_lin1_chunk_bytes(C)),
-                                         params + L.l1b + 256 * j, C, C, H, W, 256, 4 * C, 256 * j, ws.u);
-        if (rc) return rc;
+    ConvLayer cv;
+    cv.xh = ws.yh; cv.xl = ws.yl; cv.A = A; cv.C = C; cv.c_in = c4; cv.H_in = H; cv.W_in = W; cv.taps = 9;
+    cv.w = (const uint4 *)pk; cv.n_pad = conv_n_pad(c4, 32); cv.n_out = c4; cv.epi = 0; cv.out = ws.y; cv.out_ch_total = C;
+    if ((rc = conv_layer(st, cv))) return rc;
+    if ((rc = to_planes(st, ws.y, A, C, HW, ws.yh, ws.yl))) return rc;
+    // linear1 + GELU, 256 output channels (= 256 TMEM columns) per launch: the A operand is staged once per 256 columns
+    // (128 per launch was measured first: 4 x 125 us at C = 128)
+    cv.c_in = C; cv.taps = 1; cv.n_pad = cv.n_out = 256;
+    cv.epi = 2; cv.out = ws.u; cv.out_ch_total = 4 * C;
+    for (int j = 0; j < C / 64; ++j) {
+        cv.w = (const uint4 *)(pk + enh::pk_lin1_off(C) + j * enh::pk_lin1_chunk_bytes(C));
+        cv.bias = params + L.l1b + 256 * j; cv.out_ch_off = 256 * j;
+        if ((rc = conv_layer(st, cv))) return rc;
     }
     {   // depth-wise 3x3 + GELU + gate on the channel-last u, straight into linear2's bf16 operand planes
         const dim3 g3(((W + 7) / 8) * ((H + enh::kDwRows - 1) / enh::kDwRows), 2 * C / 128, A);
         enh::k_enh_dw_cl<<<g3, 256, 0, st>>>(ws.u, params, L, C, H, W, (uint2 *)ws.vh, (uint2 *)ws.vl);
         GC_LAUNCH_CHECK("k_enh_dw_cl");
     }
-    for (int j = 0; j < C / 128; ++j) {   // linear2
-        rc = enh::launch_conv<128, 1, 0>(st, grid, ws.vh, ws.vl,
-                                         (const uint4 *)(pk + enh::pk_lin2_off(C) + j * enh::pk_lin2_chunk_bytes(C)),
-                                         params + L.l2b + 128 * j, 2 * C, 2 * C, H, W, 128, C, 128 * j, ws.s);
-        if (rc) return rc;
+    // linear2
+    cv.xh = ws.vh; cv.xl = ws.vl; cv.C = cv.c_in = 2 * C; cv.n_pad = cv.n_out = 128;
+    cv.epi = 0; cv.out = ws.s; cv.out_ch_total = C;
+    for (int j = 0; j < C / 128; ++j) {
+        cv.w = (const uint4 *)(pk + enh::pk_lin2_off(C) + j * enh::pk_lin2_chunk_bytes(C));
+        cv.bias = params + L.l2b + 128 * j; cv.out_ch_off = 128 * j;
+        if ((rc = conv_layer(st, cv))) return rc;
     }
     enh::k_enh_res_gap<<<dim3(C, A), 256, 0, st>>>(ws.x1, ws.s, HW, ws.gap);
     GC_LAUNCH_CHECK("k_enh_res_gap");

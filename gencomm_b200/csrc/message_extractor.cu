@@ -32,6 +32,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "conv_layer.cuh"
 #include "implicit_gemm.cuh"
 
 namespace gc {
@@ -441,8 +442,7 @@ extern "C" int gc_message_extractor(const float *x, int total_agents, int C, int
         attr_done = true;
     }
     const dim3 grid(tiles, total_agents);
-    me::k_me_to_nhwc<<<dim3((HW + 63) / 64, C / 64, total_agents), 256, 0, st>>>(x, C, HW, ws.xh, ws.xl);
-    GC_LAUNCH_CHECK("k_me_to_nhwc");
+    if (int rc = to_planes(st, x, total_agents, C, HW, ws.xh, ws.xl)) return rc;
     if (W % me::kPix == 0 && !getenv("GC_ME_GENERIC_OFFSET")) {   // a tile is 128 pixels of one image row
         me::k_me_offset_row3<<<grid, me::kThreads, me::kR3Smem, st>>>(ws.xh, ws.xl, p_off, params + me::kOffBias, C, H, W,
                                                                       ws.offset);

@@ -578,23 +578,18 @@ def conv_planes(planes, A, c_in, H_in, W_in, packed, bias, n_out, taps, stride=1
     lib = _lib.load()
     xh, xl = planes
     Ho, Wo = ((H_in - 1) // stride + 1, (W_in - 1) // stride + 1) if taps == 9 else (H_in, W_in)
-    if out_planes is not None:
-        oh, ol = out_planes
-        _lib.check(lib.gc_conv_planes(_ptr(xh), _ptr(xl), A, c_in, H_in, W_in, stride, taps, n_out, _ptr(packed), _ptr(bias),
-                                      _ptr(oh), _ptr(ol), None, int(out_ch_total), out_ch_off, up, up_dy, up_dx, _stream()),
-                   "gc_conv_planes")
-        return out_planes, Ho, Wo
-    if out_nchw is None:
+    if out_planes is None and out_nchw is None:    # new planes of exactly this layer's output
         oh = torch.empty(max(A * Ho * Wo * n_out * 2, 1), dtype=torch.uint8, device=xh.device)
-        ol = torch.empty_like(oh)
-        _lib.check(lib.gc_conv_planes(_ptr(xh), _ptr(xl), A, c_in, H_in, W_in, stride, taps, n_out, _ptr(packed), _ptr(bias),
-                                      _ptr(oh), _ptr(ol), None, n_out, 0, 1, 0, 0, _stream()), "gc_conv_planes")
-        return (oh, ol), Ho, Wo
-    _chk(out_nchw, "out", torch.float32, 4)
-    _lib.check(lib.gc_conv_planes(_ptr(xh), _ptr(xl), A, c_in, H_in, W_in, stride, taps, n_out, _ptr(packed), _ptr(bias), None,
-                                  None, _ptr(out_nchw), out_nchw.shape[1], out_ch_off, up, up_dy, up_dx, _stream()),
-               "gc_conv_planes")
-    return None, Ho, Wo
+        out_planes = (oh, torch.empty_like(oh))
+        out_ch_total, out_ch_off, up, up_dy, up_dx = n_out, 0, 1, 0, 0
+    if out_planes is not None:
+        oh, ol, nchw = _ptr(out_planes[0]), _ptr(out_planes[1]), None
+    else:
+        _chk(out_nchw, "out", torch.float32, 4)
+        oh, ol, nchw, out_ch_total = None, None, _ptr(out_nchw), out_nchw.shape[1]
+    _lib.check(lib.gc_conv_planes(_ptr(xh), _ptr(xl), A, c_in, H_in, W_in, stride, taps, n_out, _ptr(packed), _ptr(bias), oh, ol,
+                                  nchw, int(out_ch_total), out_ch_off, up, up_dy, up_dx, _stream()), "gc_conv_planes")
+    return out_planes, Ho, Wo
 
 
 # --------------------------------------------------------------------------------------------

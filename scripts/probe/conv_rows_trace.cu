@@ -12,10 +12,13 @@ static void run(int A, int C, int NOUT, int H, int W) {
     cudaMalloc(&xh, plane); cudaMalloc(&xl, plane); cudaMalloc(&w, wbytes); cudaMalloc(&oh, obytes); cudaMalloc(&ol, obytes);
     cudaMalloc(&bias, 4096);
     cudaMemset(xh, 0x3c, plane); cudaMemset(xl, 0x30, plane); cudaMemset(w, 0x38, wbytes); cudaMemset(bias, 0, 4096);
+    gc::ConvLayer L;
+    L.xh = (const uint4 *)xh; L.xl = (const uint4 *)xl; L.A = A; L.C = L.c_in = C; L.H_in = H; L.W_in = W;
+    L.w = (const uint4 *)w; L.n_pad = L.n_out = L.out_ch_total = NOUT; L.bias = bias; L.epi = 5; L.oh = (uint4 *)oh; L.ol = (uint4 *)ol;
     cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
     for (int it = 0; it < 3; ++it) {
         cudaEventRecord(e0);
-        int rc = gc::conv_rows(0, A, xh, xl, w, bias, C, NOUT, H, W, NOUT, 0, nullptr, oh, ol);
+        int rc = gc::conv_rows(0, L);
         cudaEventRecord(e1);
         cudaError_t e = cudaDeviceSynchronize();
         if (rc || e != cudaSuccess) { printf("failed rc=%d %s\n", rc, cudaGetErrorString(e)); exit(1); }

@@ -284,7 +284,7 @@ class ConvCase:
                      emulate(op, st["x"], st["w"], st["b"], "act_residual_dropped"))
 
     def mt2(self, kind):
-        """GC_CONV_MT2=1 sends this launch to k_me_conv with two M tiles per CTA (det_tail.cu launch_layer)."""
+        """GC_CONV_MT2=1 sends this launch to k_me_conv with two M tiles per CTA (conv_layer.cu, launch)."""
         tiles = self.Ho * self.Wo // 128
         return kind == "planes" and self.taps == 9 and tiles % 2 == 0 and tiles * self.A >= 2 * 148
 
