@@ -21,7 +21,7 @@
 namespace gc {
 namespace cr {
 
-using namespace umma;
+using namespace ptx;
 using me::bf16_residual;
 
 constexpr int kStagers = 256;     // warps 0-7: operand staging (cp.async)
@@ -87,7 +87,7 @@ k_conv_rows(const uint4 *__restrict__ xh, const uint4 *__restrict__ xl, const ui
             mbar_init(smem_u32(&acc_full[i]), 1); mbar_init(smem_u32(&acc_empty[i]), kEpi);
         }
         for (int i = 0; i < NB; ++i) { mbar_init(smem_u32(&b_full[i]), 1); mbar_init(smem_u32(&b_empty[i]), 1); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     if (tid < NOUT) s_bias[tid] = bias[tid];
     tc_fence_before();

@@ -15,8 +15,6 @@
 //     tile accumulates into the other.  A CTA owns an SM for the whole launch and walks tiles b, b + gridDim.x, ...
 // Same packed weights (k_me_pack, split), same arithmetic and epilogues as k_me_conv: results are bit-identical.
 #pragma once
-#include <cuda.h>
-#include <cudaTypedefs.h>
 #include <stdlib.h>
 
 #include "implicit_gemm.cuh"
@@ -24,7 +22,7 @@
 namespace gc {
 namespace ct {
 
-using namespace umma;
+using namespace ptx;
 using me::bf16_residual;
 using me::gelu_erf;
 
@@ -58,43 +56,6 @@ __host__ __device__ constexpr int ring_depth(int NOUT, int EPI, bool STG) {
 __host__ __device__ constexpr int smem_bytes(int NOUT, int EPI, bool STG) {
     return ring_depth(NOUT, EPI, STG) * (kAStage + b_stage_bytes(NOUT)) + out_stage_bytes(NOUT, EPI, STG) + 1024;
 }
-
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap *map, int c, int x, int y, int a, uint32_t bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(c), "r"(x), "r"(y), "r"(a), "r"(bar)
-        : "memory");
-}
-__device__ __forceinline__ void bulk_copy(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src),
-                 "r"(bytes), "r"(bar)
-                 : "memory");
-}
-// the same copy delivered to the same shared-memory offset (and mbarrier) of every CTA of the cluster named in cta_mask
-__device__ __forceinline__ void bulk_copy_multicast(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar, uint16_t cta_mask) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(dst),
-        "l"(src), "r"(bytes), "r"(bar), "h"(cta_mask)
-        : "memory");
-}
-__device__ __forceinline__ void mma_commit_multicast(uint32_t bar, uint16_t cta_mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-                 "h"(cta_mask)
-                 : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// K-major SWIZZLE_64B operand: rows of 64 bytes, 8-row groups 512 bytes apart (LBO unused), layout type 4 in bits 61-63
-__device__ __forceinline__ uint64_t make_desc_sw64(uint32_t saddr) { return make_desc(saddr, 16u, 512u) | (4ull << 61); }
 
 // H x W: the output grid; tiles of BH rows x BW pixels, BW = min(W, 128), BH = 128 / BW.  stride 2: the tensor maps traverse the
 // input with element strides {1, 2, 2, 1} (box {32, 2 BW, 2 BH, 1} -> BW x BH pixels in shared memory), start (2 x0 + kx - 1, ..).
@@ -130,7 +91,7 @@ k_conv_tma(const __grid_constant__ CUtensorMap map_h, const __grid_constant__ CU
     if (tid == 32) {
         for (int i = 0; i < NS; ++i) { mbar_init(smem_u32(&full[i]), 1); mbar_init(smem_u32(&empty[i]), MC ? 2 : 1); }
         for (int i = 0; i < 2; ++i) { mbar_init(smem_u32(&acc_full[i]), 1); mbar_init(smem_u32(&acc_empty[i]), kEpi); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     for (int i = tid; i < NOUT; i += kThreads) s_bias[i] = (bias && i < n_store) ? bias[i] : 0.0f;
     tc_fence_before();
@@ -313,23 +274,10 @@ k_conv_tma(const __grid_constant__ CUtensorMap map_h, const __grid_constant__ CU
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-inline PFN_cuTensorMapEncodeTiled_v12000 get_encode() {
-    static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(p);
-        (void)cudaGetLastError();
-    }
-    return fn;
-}
 // planes [A][H][W][C] bf16 as the 4-D tensor (C, W, H, A); box = {32 channels, BW, BH, 1} output pixels, 64-byte swizzle, zero fill
 // outside; H x W is the INPUT grid, every stride-th pixel is loaded
 inline bool encode_plane_map(CUtensorMap *map, const void *plane, int A, int H, int W, int C, int BW, int BH, int stride) {
-    PFN_cuTensorMapEncodeTiled_v12000 encode = get_encode();
+    const auto encode = tensor_map_encoder();
     if (!encode) return false;
     const cuuint64_t gdim[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)A};
     const cuuint64_t gstride[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};

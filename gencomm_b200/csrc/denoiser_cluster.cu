@@ -27,13 +27,13 @@
 #include "common.cuh"
 #include "denoiser_cluster.cuh"
 #include "denoiser_tc.cuh"
-#include "umma.cuh"
+#include "ptx.cuh"
 
 namespace gc {
 namespace cl {
 
 namespace cg = cooperative_groups;
-using namespace umma;
+using namespace ptx;
 
 constexpr int kStageWarps = 16;                    // staging + epilogue warps
 constexpr int kStageThreads = kStageWarps * 32;    // 512
@@ -119,9 +119,6 @@ __device__ __forceinline__ float4 ld_cluster4(uint32_t caddr) {
     asm volatile("ld.shared::cluster.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(caddr));
     return v;
 }
-__device__ __forceinline__ void st_cluster(uint32_t caddr, float v) {
-    asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(caddr), "f"(v) : "memory");
-}
 __device__ __forceinline__ float4 lds4(uint32_t saddr) {
     float4 v;
     asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(saddr));
@@ -130,95 +127,17 @@ __device__ __forceinline__ float4 lds4(uint32_t saddr) {
 __device__ __forceinline__ void sts4(uint32_t saddr, float4 v) {
     asm volatile("st.shared.v4.f32 [%0], {%1,%2,%3,%4};" ::"r"(saddr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
 }
-
-// ---- tensor memory ----
-__device__ __forceinline__ void tmem_alloc512(uint32_t *slot) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(slot)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_free512(uint32_t base) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(base) : "memory");
-}
-__device__ __forceinline__ void tmem_zero8(uint32_t taddr) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%1,%1,%1,%1,%1,%1,%1};" ::"r"(taddr), "r"(0u) : "memory");
-}
-__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void tmem_ld16_nowait(uint32_t taddr, float *v) {
-    uint32_t r[16];
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr));
-#pragma unroll
-    for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
-__host__ __device__ constexpr uint32_t make_idesc_tf32(int M, int N) {
-    return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-__device__ __forceinline__ void mma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t"
-        "}" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-
 __device__ __forceinline__ float lds1(uint32_t saddr) {
     float v;
     asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(saddr));
     return v;
 }
 __device__ __forceinline__ void sts1(uint32_t saddr, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(saddr), "f"(v) : "memory"); }
-__device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
-__device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory"); }
 __device__ __forceinline__ void stage_bar() { asm volatile("bar.sync 1, %0;" ::"n"(kStageThreads) : "memory"); }   // staging warps only
 
-// Remote 16-byte store whose completion is counted (in bytes) on an mbarrier of the destination CTA: the data is visible
-// to whoever observes the barrier phase complete -- no cluster-scope fence on the producer.  The hardware cluster
-// barrier costs MEMBAR.ALL.GPU + ERRBAR on every arrive.release (measured 1400 cycles per layer, profiles/r02i_trace.txt).
-__device__ __forceinline__ void st_async4(uint32_t remote_addr, float4 v, uint32_t remote_bar) {
-    asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.f32 [%0], {%1,%2,%3,%4}, [%5];"
-                 ::"r"(remote_addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w), "r"(remote_bar) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-// Issued inside an `if (elect_one())` branch of a converged warp with operands derived from kernel parameters, constants
-// and loop counters only: ptxas then keeps the descriptors in uniform registers (UIADD3 + UTCHMMA, 3 instructions per MMA).
-// Predicating every MMA on its own elect.sync, or branching on tid == 0, costs 5 R2UR per MMA (~100 cycles each measured).
-__device__ __forceinline__ void mma_tf32_plain(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred pa;\n\t"
-        "setp.ne.b32 pa, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, pa;\n\t"
-        "}" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-
-// x * sigmoid(x) = h + h * tanh(h), h = x / 2: one MUFU per element (tanh.approx, rel. error 2^-11 = the tf32 operand grid)
-__device__ __forceinline__ float swish_tanh(float u) {
-    const float h = 0.5f * u;
-    float t;
-    asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(h));
-    return fmaf(h, t, h);
-}
-
-// two activations per MUFU: tanh.approx.f16x2 (|tanh| <= 1 in fp16: absolute error 2^-11, the tf32 operand grid).  The
+// x * sigmoid(x) = h + h * tanh(h) with h = x / 2 already formed (the GroupNorm coefficients are stored pre-halved), two
+// activations per MUFU: tanh.approx.f16x2 (|tanh| <= 1 in fp16: absolute error 2^-11, the tf32 operand grid).  The
 // staging pass is MUFU bound (10.4 k activations per layer and CTA at 16 / clock, profiles/r02j_cluster_trace_v3.txt).
-__device__ __forceinline__ void swish_tanh2(float &u0, float &u1) {
-    const float h0 = 0.5f * u0, h1 = 0.5f * u1;
-    const __half2 hh = __floats2half2_rn(h0, h1);
-    uint32_t t;
-    asm("tanh.approx.f16x2 %0, %1;" : "=r"(t) : "r"(*reinterpret_cast<const uint32_t *>(&hh)));
-    const float2 tf = __half22float2(*reinterpret_cast<const __half2 *>(&t));
-    u0 = fmaf(h0, tf.x, h0);
-    u1 = fmaf(h1, tf.y, h1);
-}
-
-// the same with h = x / 2 already formed (the GroupNorm coefficients are stored pre-halved)
 __device__ __forceinline__ void swish_half2(float &h0, float &h1) {
     const __half2 hh = __floats2half2_rn(h0, h1);
     uint32_t t;
@@ -476,8 +395,8 @@ __device__ __forceinline__ void mma_layer(Ctx &c, uint32_t rec_saddr) {
                 for (int cg = 0; cg < CG; ++cg) {
 #pragma unroll
                     for (int kx = 0; kx < 3; ++kx)   // +1 in the address field = one 16-byte pixel; B: 2048 B per kx, 1024 B per group
-                        mma_tf32_plain(kTmem + 8u * i, a_base + (uint64_t)(cg * 2 * (kPlane / 16u) + slot * kRowPx + kx),
-                                       b_base + (uint64_t)(kx * 128 + cg * 64), idesc, 1u);
+                        mma_tf32(kTmem + 8u * i, a_base + (uint64_t)(cg * 2 * (kPlane / 16u) + slot * kRowPx + kx),
+                                 b_base + (uint64_t)(kx * 128 + cg * 64), idesc, 1u);
                 }
             }
         }
@@ -519,15 +438,9 @@ __device__ __forceinline__ void epilogue_layer(Ctx &c, const LayerCfg &L, uint32
         if (px >= PXW || hsel >= R / 2) continue;      // warp-uniform (half resolution: 4 of the 16 warps work)
         const int r0 = ph * (R / 2) + hsel;
         float a[8];
-        {
-            uint32_t rr[8];
-            asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                         : "=r"(rr[0]), "=r"(rr[1]), "=r"(rr[2]), "=r"(rr[3]), "=r"(rr[4]), "=r"(rr[5]), "=r"(rr[6]), "=r"(rr[7])
-                         : "r"(kTmem + ((uint32_t)(q * 32) << 16) + 8u * (r0 + 2)));
-            tmem_wait_ld();
+        tmem_ld8(kTmem + ((uint32_t)(q * 32) << 16) + 8u * (r0 + 2), a);
 #pragma unroll
-            for (int i = 0; i < 8; ++i) a[i] = __uint_as_float(rr[i]) + bias[i];
-        }
+        for (int i = 0; i < 8; ++i) a[i] += bias[i];
         const uint32_t poff = (uint32_t)((r0 * 2) * PXW + px) * 16u;
         if (L.res != kNone) {
             const float4 a0 = lds4(ra_base + poff), a1 = lds4(ra_base + poff + PXW * 16u);
@@ -698,7 +611,7 @@ k_unet_middle_cluster(const float *__restrict__ h0, const float *__restrict__ re
     const int n_clusters = gridDim.x / kCl, cluster_id = blockIdx.x / kCl;
     Misc *misc = reinterpret_cast<Misc *>(smem_raw + kOffMisc);
 
-    if (c.warp == 0) tmem_alloc512(&misc->tmem);
+    if (c.warp == 0) tmem_alloc<512>(&misc->tmem);
     if (c.tid == 32) {
         for (int i = 0; i < 3; ++i) mbar_init(MISC_ADDR(c, pass_bar) + 8u * i, kStageWarps);
         for (int i = 0; i < 2; ++i) mbar_init(MISC_ADDR(c, free_bar) + 8u * i, 1);
@@ -706,7 +619,7 @@ k_unet_middle_cluster(const float *__restrict__ h0, const float *__restrict__ re
             mbar_init(MISC_ADDR(c, done_bar) + 8u * i, 1); mbar_init(MISC_ADDR(c, rec_bar) + 8u * i, 1);
             mbar_init(MISC_ADDR(c, sync_bar) + 8u * i, 1);
         }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
         mbar_expect_tx(MISC_ADDR(c, sync_bar), kCl * 32u);          // hand-overs 0 and 1
         mbar_expect_tx(MISC_ADDR(c, sync_bar) + 8u, kCl * 32u);
     }
@@ -762,7 +675,7 @@ k_unet_middle_cluster(const float *__restrict__ h0, const float *__restrict__ re
     __syncthreads();
     cluster_arrive();                                   // no CTA exits while a peer may still push into its shared memory
     cluster_wait();
-    if (c.warp == 0) tmem_free512(kTmem);
+    if (c.warp == 0) tmem_free<512>(kTmem);
 }
 
 }  // namespace cl

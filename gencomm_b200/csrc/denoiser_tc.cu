@@ -22,22 +22,13 @@
 
 #include "common.cuh"
 #include "denoiser_tc.cuh"
-#include "umma.cuh"
+#include "ptx.cuh"
 
 namespace gc {
 namespace tc {
 
-using namespace umma;
+using namespace ptx;
 
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
-    uint32_t r[8];
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-                 : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-    for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
-}
 __device__ __forceinline__ uint4 pack8(const float (&v)[8]) {
     return make_uint4(pack_bf16(v[0], v[1]), pack_bf16(v[2], v[3]), pack_bf16(v[4], v[5]), pack_bf16(v[6], v[7]));
 }
@@ -124,7 +115,7 @@ k_conv_out_tc(const float *__restrict__ in, const float *__restrict__ st_in, int
     const int x0 = blockIdx.x * 128, y_first = blockIdx.y * kOutRows;
 
     if (warp == 0) tmem_alloc<NT>(&s_tmem);
-    if (tid == 32) { mbar_init(smem_u32(&s_bar), 1); asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
+    if (tid == 32) { mbar_init(smem_u32(&s_bar), 1); mbar_init_fence(); }
     if (tid >= 64 && tid < 72) {
         const int c = tid - 64;
         gn_coeff8(c, agent, st_in, tiles_in, H * W, aff.gamma[c], aff.beta[c], &s_ga[c], &s_gb[c]);
@@ -262,7 +253,7 @@ k_conv_in_tc(const float *__restrict__ cond, const float *__restrict__ x, const 
     if (warp == 0) tmem_alloc<64>(&s_tmem);
     if (tid == 32) {
         mbar_init(smem_u32(&s_empty[0]), 1); mbar_init(smem_u32(&s_empty[1]), 1); mbar_init(smem_u32(&s_done), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     // ---- B operand for every chunk: pre-packed [q][tap][gsel][n][8 bf16] ----
     for (int i = tid; i < chunks * 9 * 2 * 8; i += 128) b_s[i] = __ldg(wp + i);
@@ -409,24 +400,6 @@ __global__ void k_pack_conv_in_w2(const float *__restrict__ w, int C, int chunks
     out[i] = pack8(f);
 }
 
-__device__ __forceinline__ void mma_bf16_elect(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred pe, pa;\n\t"
-        "setp.eq.b32 pa, 0, 0;\n\t"
-        "elect.sync _|pe, 0xffffffff;\n\t"
-        "@pe tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, pa;\n\t"
-        "}" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc) : "memory");
-}
-__device__ __forceinline__ void commit_elect(uint32_t bar) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred pe;\n\t"
-        "elect.sync _|pe, 0xffffffff;\n\t"
-        "@pe tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n\t"
-        "}" ::"r"(bar) : "memory");
-}
-
 __global__ void __launch_bounds__(kIn2Threads)
 k_conv_in_tc2(const float *__restrict__ cond, const float *__restrict__ x, const uint4 *__restrict__ wp2, Bias8 bias, int C, int H,
               int W, float *__restrict__ out, float *__restrict__ stats_out) {
@@ -448,7 +421,7 @@ k_conv_in_tc2(const float *__restrict__ cond, const float *__restrict__ x, const
     if (tid == 32) {
         mbar_init(smem_u32(&s_empty[0]), 1); mbar_init(smem_u32(&s_empty[1]), 1); mbar_init(smem_u32(&s_done), 1);
         mbar_init(smem_u32(&s_wbar), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     // x halo columns (pixels -1 and 128) are outside the image for W == 128: zero once, staging never touches them
     for (int i = tid; i < 2 * 2 * kIn2Staged * 2; i += kIn2Threads) {
@@ -464,8 +437,8 @@ k_conv_in_tc2(const float *__restrict__ cond, const float *__restrict__ x, const
         const uint32_t ta = tmem + ((uint32_t)(warp * 32) << 16);
 #pragma unroll
         for (int j = 0; j < 13; ++j)
-            asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%1,%1,%1,%1,%1,%1,%1};" ::"r"(ta + 8u * j), "r"(0u) : "memory");
-        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+            tmem_zero8(ta + 8u * j);
+        tmem_wait_st();
     }
     const uint32_t a_base = smem_u32(a_s), b_base = smem_u32(b_s);
     constexpr uint32_t idesc = make_idesc(128, 32);
@@ -583,18 +556,6 @@ k_conv_in_tc2(const float *__restrict__ cond, const float *__restrict__ x, const
 // zero AFTER the activation); bias / timestep embedding, the residual or the 1x1 nin_shortcut and the GroupNorm
 // partial sums of the output are the epilogue.  N = 16 with SBO = 0 on B (columns 8..15 alias 0..7, ignored).
 // ------------------------------------------------------------------------------------------------
-__host__ __device__ constexpr uint32_t make_idesc_tf32(int M, int N) {
-    return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-__device__ __forceinline__ void mma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t"
-        "}" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-
 constexpr int kMidRows = 4, kMidStaged = kMidRows + 2, kMidRowPx = 130;
 constexpr int kMidPlaneU4 = kMidStaged * kMidRowPx;   // uint4 (16-byte pixel halves) per plane
 
@@ -618,7 +579,7 @@ k_conv_c8_tc(const float *__restrict__ in_a, const float *__restrict__ in_b, con
     const int Hin = GEOM == kUp ? H / 2 : H, Win = GEOM == kUp ? W / 2 : W;
 
     if (warp == 0) tmem_alloc<kMidRows * 16 <= 32 ? 32 : 64>(&s_tmem);
-    if (tid == 32) { mbar_init(smem_u32(&s_done), 1); asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
+    if (tid == 32) { mbar_init(smem_u32(&s_done), 1); mbar_init_fence(); }
     if (PRE_GN && tid >= 64 && tid < 64 + CIN) {
         // GroupNorm(4 groups) coefficients from per-tile partial sums (same fixed-order float64 combination as
         // gn_coeff<CIN> in denoiser.cu): CIN == 8: one channel pair per group; CIN == 16: two pairs of one tensor

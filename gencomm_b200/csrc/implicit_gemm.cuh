@@ -7,12 +7,12 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
-#include "umma.cuh"
+#include "ptx.cuh"
 
 namespace gc {
 namespace me {
 
-using namespace umma;
+using namespace ptx;
 
 constexpr int kPix = 128;            // pixels per CTA = M
 constexpr int kThreads = 256;          // threads that stage operands and run the epilogue
@@ -169,7 +169,7 @@ k_me_conv(const uint4 *__restrict__ xh, const uint4 *__restrict__ xl, const floa
         mbar_init(smem_u32(&s_empty[0]), 1); mbar_init(smem_u32(&s_empty[1]), 1); mbar_init(smem_u32(&s_done), 1);
         mbar_init(smem_u32(&s_full[0]), 1); mbar_init(smem_u32(&s_full[1]), 1);
         mbar_init(smem_u32(&s_afull[0]), kThreads); mbar_init(smem_u32(&s_afull[1]), kThreads);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     tc_fence_before();
     __syncthreads();

@@ -69,7 +69,7 @@ k_me_offset_row3(const uint4 *__restrict__ xh, const uint4 *__restrict__ xl, con
     if (warp == 0) tmem_alloc<NOUT>(&s_tmem);
     if (tid == 32) {
         mbar_init(smem_u32(&s_empty[0]), 1); mbar_init(smem_u32(&s_empty[1]), 1); mbar_init(smem_u32(&s_done), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     tc_fence_before();
     __syncthreads();
@@ -272,7 +272,7 @@ k_me_tail_tc(const float *__restrict__ b1, const float *__restrict__ attn, const
     if (warp == 0) tmem_alloc<64>(&s_tmem);
     if (tid == 32) {
         mbar_init(smem_u32(&s_done), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     if (tid < 64) {
         s_attn[tid] = attn[a * 64 + tid];

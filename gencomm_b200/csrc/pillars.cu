@@ -23,13 +23,14 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "ptx.cuh"
 
-#include <cuda.h>
-#include <cudaTypedefs.h>
 #include <stdlib.h>
 #include <string.h>
 
 namespace gc {
+
+using namespace ptx;
 
 // ------------------------------------------------------------------------------------------------
 // agent lookup: largest a with off[a] <= g
@@ -968,39 +969,6 @@ struct CvSmem {
     int dirty[NB];
 };
 
-__device__ __forceinline__ uint32_t cv_smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void cv_mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void cv_mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void cv_mbar_wait(uint32_t bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "CV_WAIT_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra CV_DONE_%=;\n\t"
-        "bra CV_WAIT_%=;\n\t"
-        "CV_DONE_%=:\n\t}" ::"r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ bool cv_mbar_test(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}" : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void cv_fence_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void cv_tma_store_box(const CUtensorMap *map, uint32_t src, int x, int y, int plane) {
-    asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%1, %2, %3}], [%4];"
-                 ::"l"(reinterpret_cast<uint64_t>(map)), "r"(x), "r"(y), "r"(plane), "r"(src) : "memory");
-}
-__device__ __forceinline__ void cv_bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void cv_bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void cv_bulk_wait_read1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
-
 struct PfnPacked {
     float a0a, a1a, a2a, a3a;    // channel `lane`      (FFMA2 takes a scalar multiplier for both halves)
     float a0b, a1b, a2b, a3b;    // channel `lane + 32`
@@ -1107,7 +1075,7 @@ k_canvas_persist(const __grid_constant__ CUtensorMap tmap, const FusedSrc src, c
     static_assert(kCvLists > NB && (kCvLists & (kCvLists - 1)) == 0, "list ring");
     extern __shared__ __align__(1024) unsigned char cv_smem_raw[];   // 1024-byte alignment: swizzled TMA boxes
     Smem &sm = *reinterpret_cast<Smem *>(cv_smem_raw);
-    if ((cv_smem_u32(cv_smem_raw) & 1023u) != 0u) __trap();
+    if ((smem_u32(cv_smem_raw) & 1023u) != 0u) __trap();
     const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
     const int tiles_x = (nx + kTileX - 1) / kTileX;
     const int total_tiles = n_agents * ny * tiles_x;
@@ -1132,16 +1100,16 @@ k_canvas_persist(const __grid_constant__ CUtensorMap tmap, const FusedSrc src, c
     }
     if (t == 0) {
         for (int s = 0; s < NB; ++s) {
-            cv_mbar_init(cv_smem_u32(&sm.full[s]), W);
-            cv_mbar_init(cv_smem_u32(&sm.empty[s]), 1);
+            mbar_init(smem_u32(&sm.full[s]), W);
+            mbar_init(smem_u32(&sm.empty[s]), 1);
             sm.dirty[s] = 0;
         }
-        for (int s = 0; s < kCvLists; ++s) cv_mbar_init(cv_smem_u32(&sm.ready[s]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        for (int s = 0; s < kCvLists; ++s) mbar_init(smem_u32(&sm.ready[s]), 1);
+        mbar_init_fence();
     }
     __syncthreads();
-    const uint32_t full0 = cv_smem_u32(&sm.full[0]), empty0 = cv_smem_u32(&sm.empty[0]);
-    const uint32_t ready0 = cv_smem_u32(&sm.ready[0]), take0 = cv_smem_u32(&sm.list_take[0]);
+    const uint32_t full0 = smem_u32(&sm.full[0]), empty0 = smem_u32(&sm.empty[0]);
+    const uint32_t ready0 = smem_u32(&sm.ready[0]), take0 = smem_u32(&sm.list_take[0]);
 
     if (warp == W) {
         // ------------------------------ control warp ----------------------------------------------
@@ -1188,7 +1156,7 @@ k_canvas_persist(const __grid_constant__ CUtensorMap tmap, const FusedSrc src, c
             put(o3, c.w, 3);
             if (lane == 31) { sm.list_n[slot] = incl; sm.list_pbase[slot] = lt_pbase; sm.list_take[slot] = 0; }
             __syncwarp();
-            if (lane == 0) cv_mbar_arrive(ready0 + 8u * slot);
+            if (lane == 0) mbar_arrive(ready0 + 8u * slot);
             ++lt_i;
             if (lt_i < n_my) { lt.advance(step, ny, tiles_x); codes = load_codes(lt); }
         };
@@ -1208,39 +1176,39 @@ k_canvas_persist(const __grid_constant__ CUtensorMap tmap, const FusedSrc src, c
                 if (lane == 0) sm.dirty[rb] = 0;
             }
             __syncwarp();
-            if (lane == 0) cv_mbar_arrive(empty0 + 8u * rb);
+            if (lane == 0) mbar_arrive(empty0 + 8u * rb);
         };
         int prev = -1;
 #pragma unroll 1
         for (int i = 0; i < n_my; ++i) {
-            cv_mbar_wait(full0 + 8u * buf, parity);   // every PFN warp is done with tile i and with list i
-            cv_fence_async();
+            mbar_wait(full0 + 8u * buf, parity);   // every PFN warp is done with tile i and with list i
+            fence_async_smem();
             if (lane == 0) {   // four [32 cells][64 channels] boxes; the part of a box beyond nx is clipped by the TMA unit
                 const int x0 = it.tx * kTileX;
-                const uint32_t s_box = cv_smem_u32(&sm.tile[buf][0]);
+                const uint32_t s_box = smem_u32(&sm.tile[buf][0]);
 #pragma unroll
                 for (int k = 0; k < 4; ++k)
-                    if (x0 + 32 * k < nx) cv_tma_store_box(&tmap, s_box + 8192u * k, x0 + 32 * k, it.y, it.b * 64);
-                cv_bulk_commit();
+                    if (x0 + 32 * k < nx) tma_store_box(&tmap, s_box + 8192u * k, x0 + 32 * k, it.y, it.b * 64);
+                bulk_commit();
             }
             if (lt_i < n_my) build_list();            // reuses the ring slot of list i; overlaps the bulk reads
             // the shared-memory reads of tile i overlap the next iteration: only tile i - 1 is reclaimed here
             if (PIPE) {
                 if (prev >= 0) {
-                    if (lane == 0) cv_bulk_wait_read1();
+                    if (lane == 0) bulk_wait_read<1>();
                     __syncwarp();
                     release(prev);
                 }
                 prev = buf;
             } else {
-                if (lane == 0) cv_bulk_wait_read();
+                if (lane == 0) bulk_wait_read<0>();
                 __syncwarp();
                 release(buf);
             }
             it.advance(step, ny, tiles_x);
             if (++buf == NB) { buf = 0; parity ^= 1u; }
         }
-        if (lane == 0) cv_bulk_wait_read();   // shared memory must outlive the last reads
+        if (lane == 0) bulk_wait_read<0>();   // shared memory must outlive the last reads
         __syncwarp();
         return;
     }
@@ -1292,7 +1260,7 @@ k_canvas_persist(const __grid_constant__ CUtensorMap tmap, const FusedSrc src, c
                 }
                 if (g_i >= n_my - 1) { g_i = n_my; s.i = -1; return; }
                 const int slot = (g_i + 1) & (kCvLists - 1);
-                if (!cv_mbar_test(ready0 + 8u * slot, (uint32_t)((g_i + 1) / kCvLists) & 1u)) { s.i = g_i + 1; return; }
+                if (!mbar_test(ready0 + 8u * slot, (uint32_t)((g_i + 1) / kCvLists) & 1u)) { s.i = g_i + 1; return; }
                 ++g_i;
                 g_n = sm.list_n[slot];
                 g_pbase = sm.list_pbase[slot];
@@ -1314,14 +1282,14 @@ k_canvas_persist(const __grid_constant__ CUtensorMap tmap, const FusedSrc src, c
             while (cur_i < target) {
                 if (wrote) {
                     if (lane == 0) sm.dirty[cur_buf] = 1;
-                    cv_fence_async();
+                    fence_async_smem();
                     wrote = false;
                 }
                 __syncwarp();
-                if (lane == 0) cv_mbar_arrive(full0 + 8u * cur_buf);
+                if (lane == 0) mbar_arrive(full0 + 8u * cur_buf);
                 ++cur_i;
                 if (++cur_buf == NB) { cur_buf = 0; cur_par ^= 1u; }
-                if (cur_i < n_my) cv_mbar_wait(empty0 + 8u * cur_buf, cur_par);
+                if (cur_i < n_my) mbar_wait(empty0 + 8u * cur_buf, cur_par);
             }
         };
         auto pipe = [&](Slot &s0, Slot &s1, Slot &s2) {
@@ -1462,7 +1430,7 @@ k_canvas_persist(const __grid_constant__ CUtensorMap tmap, const FusedSrc src, c
             }
             if (g_i >= n_my - 1) { g_i = n_my; s.e = CvEnt{-1, -1, 0}; return; }
             const int slot = (g_i + 1) & (kCvLists - 1);
-            if (!cv_mbar_test(ready0 + 8u * slot, (uint32_t)((g_i + 1) / kCvLists) & 1u)) {
+            if (!mbar_test(ready0 + 8u * slot, (uint32_t)((g_i + 1) / kCvLists) & 1u)) {
                 s.e = CvEnt{g_i + 1, -1, 0};
                 return;
             }
@@ -1485,14 +1453,14 @@ k_canvas_persist(const __grid_constant__ CUtensorMap tmap, const FusedSrc src, c
         while (cur_i < target) {
             if (wrote) {
                 if (lane == 0) sm.dirty[cur_buf] = 1;
-                cv_fence_async();
+                fence_async_smem();
                 wrote = false;
             }
             __syncwarp();
-            if (lane == 0) cv_mbar_arrive(full0 + 8u * cur_buf);
+            if (lane == 0) mbar_arrive(full0 + 8u * cur_buf);
             ++cur_i;
             if (++cur_buf == NB) { cur_buf = 0; cur_par ^= 1u; }
-            if (cur_i < n_my) cv_mbar_wait(empty0 + 8u * cur_buf, cur_par);
+            if (cur_i < n_my) mbar_wait(empty0 + 8u * cur_buf, cur_par);
         }
     };
     // one pipeline step: s0 is evaluated, s1 gets its points, s2 becomes the pillar after s1
@@ -1543,24 +1511,9 @@ k_build_cell_map(const int4 *__restrict__ coords, int n_pillars, int nx, int ny,
     cell_map[(size_t)c.x * nx * ny + idx] = m;
 }
 
-static PFN_cuTensorMapEncodeTiled_v12000 cv_get_encode() {
-    static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-            q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(p);
-        (void)cudaGetLastError();
-    }
-    return fn;
-}
-
 // canvas [A*64][ny][nx] f32 as a 3-D tensor; box = 32 cells x 1 row x 64 channel planes, 128-byte swizzle in shared memory
 static bool cv_encode_map(CUtensorMap *map, float *canvas, int nx, int ny, long long planes) {
-    PFN_cuTensorMapEncodeTiled_v12000 encode = cv_get_encode();
+    const auto encode = tensor_map_encoder();
     if (!encode) return false;
     const cuuint64_t gdim[3] = {(cuuint64_t)nx, (cuuint64_t)ny, (cuuint64_t)planes};
     const cuuint64_t gstride[2] = {(cuuint64_t)nx * 4, (cuuint64_t)ny * nx * 4};

@@ -5,11 +5,39 @@
 // (models/sub_modules/torch_transformation_utils.py:329-331).  Unnormalisation, floor, the four weights and
 // the tap accumulation order follow ATen's grid_sampler_2d CUDA kernel (align_corners=False, zeros padding).
 #pragma once
+#include <type_traits>
+#include <utility>
+
 #include "common.cuh"
 
 namespace gc {
 
 constexpr int kMaxN = GC_MAX_AGENTS_PER_FRAME;
+
+// ---- helpers of the TMA-staged kernels (warp_fuse_tile.cu, warp_fuse_persist.cu) ----
+template <int kCount>
+__device__ __forceinline__ void consumer_sync() {   // named barrier 1: consumer warps only
+    asm volatile("bar.sync 1, %0;" ::"n"(kCount) : "memory");
+}
+// shared-memory accesses by 32-bit shared address + compile-time byte offset (folds into the LDS/STS immediate)
+template <int OFF>
+__device__ __forceinline__ float lds(uint32_t addr) {
+    float v;
+    asm volatile("ld.shared.f32 %0, [%1+%2];" : "=f"(v) : "r"(addr), "n"(OFF));
+    return v;
+}
+template <int OFF>
+__device__ __forceinline__ void sts(uint32_t addr, float v) {
+    asm volatile("st.shared.f32 [%0+%1], %2;" ::"r"(addr), "n"(OFF), "f"(v) : "memory");
+}
+template <int... Is, class F>
+__device__ __forceinline__ void static_for_impl(std::integer_sequence<int, Is...>, F &&f) {
+    (f(std::integral_constant<int, Is>{}), ...);
+}
+template <int N, class F>
+__device__ __forceinline__ void static_for(F &&f) {   // f(std::integral_constant<int, i>) for i = 0 .. N-1
+    static_for_impl(std::make_integer_sequence<int, N>{}, static_cast<F &&>(f));
+}
 
 // ATen linspace(-1,1,n) * (n-1)/n, evaluated in float64 (AffineGridGenerator.cpp: linspace_from_neg_one).
 __host__ __device__ __forceinline__ double base_coord(int i, int n) {

@@ -26,17 +26,15 @@
 // Requirements checked by the host: W % 4 == 0 and 16-byte aligned base (TMA global strides; the probe
 // scripts/probes/tma_align.cu shows the innermost TMA start coordinate must be a multiple of 16 bytes), at most
 // kTileMaxN agents per frame.  Otherwise gc_warp_fuse uses the gather kernels of warp_fuse.cu.
-#include <cuda.h>
-#include <cudaTypedefs.h>
 #include <stdlib.h>
 
-#include <type_traits>
-#include <utility>
-
+#include "ptx.cuh"
 #include "warp_common.cuh"
 
 namespace gc {
 namespace persist {
+
+using namespace ptx;
 
 constexpr int kTileMaxN = 8;
 constexpr int kMaxStages = 8;
@@ -69,90 +67,6 @@ struct Cfg {
     static_assert(kConsumers % 32 == 0, "whole consumer warps");
     static_assert(kThreads <= 1024, "block too large");
 };
-
-// ---- PTX wrappers -----------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "WAIT_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra DONE_%=;\n\t"
-        "bra WAIT_%=;\n\t"
-        "DONE_%=:\n\t"
-        "}" ::"r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void tma_load_box(uint32_t dst, const CUtensorMap *map, int x, int y, int plane, uint32_t bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(x), "r"(y), "r"(plane), "r"(bar)
-        : "memory");
-}
-template <int kCount>
-__device__ __forceinline__ void consumer_sync() {   // named barrier 1: consumer warps only
-    asm volatile("bar.sync 1, %0;" ::"n"(kCount) : "memory");
-}
-template <int OFF>
-__device__ __forceinline__ float lds(uint32_t addr) {
-    float v;
-    asm volatile("ld.shared.f32 %0, [%1+%2];" : "=f"(v) : "r"(addr), "n"(OFF));
-    return v;
-}
-template <int OFF>
-__device__ __forceinline__ void sts(uint32_t addr, float v) {
-    asm volatile("st.shared.f32 [%0+%1], %2;" ::"r"(addr), "n"(OFF), "f"(v) : "memory");
-}
-// ---- tensor memory as a 256 KB per-SM scratchpad (AttFusion park): lane = pixel % 128, column = (agent, channel) ----
-__device__ __forceinline__ void tmem_alloc_all(uint32_t *slot) {   // one full warp; all 512 columns (1 CTA per SM)
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(slot)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_free_all(uint32_t base) {     // the same warp
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(base) : "memory");
-}
-__device__ __forceinline__ void tmem_st4(uint32_t taddr, float a, float b, float c, float d) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};" ::"r"(taddr), "r"(__float_as_uint(a)),
-                 "r"(__float_as_uint(b)), "r"(__float_as_uint(c)), "r"(__float_as_uint(d)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
-    uint32_t r[8];
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-                 : "r"(taddr));
-#pragma unroll
-    for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
-    uint32_t r[16];
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr));
-#pragma unroll
-    for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-
-template <int... Is, class F>
-__device__ __forceinline__ void static_for_impl(std::integer_sequence<int, Is...>, F &&f) {
-    (f(std::integral_constant<int, Is>{}), ...);
-}
-template <int N, class F>
-__device__ __forceinline__ void static_for(F &&f) {
-    static_for_impl(std::make_integer_sequence<int, N>{}, static_cast<F &&>(f));
-}
 
 struct TapS {
     float w_nw, w_ne, w_sw, w_se;
@@ -386,8 +300,8 @@ __device__ __forceinline__ void fast_loop(Ctx &x, const float (&wt)[kTileMaxN][4
             int c = 0;
             for (; c + 8 <= x.C; c += 8) {
                 float pa[16], pb[16], ea[4] = {0.f, 0.f, 0.f, 0.f}, eb[4] = {0.f, 0.f, 0.f, 0.f};
-                tmem_ld16(x.tmem_park + (uint32_t)(c * 4), pa);
-                tmem_ld16(x.tmem_park + (uint32_t)(c * 4 + 16), pb);
+                tmem_ld16_nowait(x.tmem_park + (uint32_t)(c * 4), pa);
+                tmem_ld16_nowait(x.tmem_park + (uint32_t)(c * 4 + 16), pb);
                 if (IDENT0 && !kEgoCol) {
 #pragma unroll
                     for (int i = 0; i < 4; ++i) {
@@ -402,7 +316,7 @@ __device__ __forceinline__ void fast_loop(Ctx &x, const float (&wt)[kTileMaxN][4
             }
             for (; c < x.C; c += 4) {   // C % 4 == 0 in this mode
                 float pv[16], ego[4] = {0.f, 0.f, 0.f, 0.f};
-                tmem_ld16(x.tmem_park + (uint32_t)(c * 4), pv);
+                tmem_ld16_nowait(x.tmem_park + (uint32_t)(c * 4), pv);
                 if (IDENT0 && !kEgoCol) {
 #pragma unroll
                     for (int i = 0; i < 4; ++i) ego[i] = x.active ? __ldg(sp + (size_t)i * x.plane) : 0.0f;
@@ -562,12 +476,13 @@ k_fuse_persist(const __grid_constant__ CUtensorMap tmap_box, const __grid_consta
     if (tid == 0) {
         for (int s = 0; s < kMaxStages; ++s) { mbar_init(full_addr + 8u * s, 1); mbar_init(empty_addr + 8u * s, kConsumers / 32); }
         for (int s = 0; s < kGeomSlots; ++s) { mbar_init(gfull_addr + 8u * s, 1); mbar_init(gempty_addr + 8u * s, kConsumers / 32 + 1); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
-    if (MODE == GC_FUSE_ATT && plan.park_tmem && tid < 32) tmem_alloc_all(&s_tmem);
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    // tensor memory as a 256 KB per-SM scratchpad (AttFusion park, lane = pixel % 128): all 512 columns, 1 CTA per SM
+    if (MODE == GC_FUSE_ATT && plan.park_tmem && tid < 32) tmem_alloc<512>(&s_tmem);
+    tc_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tc_fence_after();
 
     // ---- geometry warp: box origins / paths of the tiles ahead, published through a small ring so that neither the
     // producer nor the consumers have the float64 corner evaluation (and the per-tile identity check) on their path
@@ -715,32 +630,17 @@ k_fuse_persist(const __grid_constant__ CUtensorMap tmap_box, const __grid_consta
 #undef GC_FAST
     }
     if (MODE == GC_FUSE_ATT && plan.park_tmem) {   // every consumer is done with tensor memory
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tc_fence_before();
         consumer_sync<kConsumers>();
-        if (tid < 32) tmem_free_all(s_tmem);
+        if (tid < 32) tmem_free<512>(s_tmem);
     }
 }
 
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-static PFN_cuTensorMapEncodeTiled_v12000 get_encode() {
-    static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-            q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(p);
-        (void)cudaGetLastError();
-    }
-    return fn;
-}
-
 static bool encode_map(CUtensorMap *map, const float *feat, int W, int H, long long planes, int bw, int bh, int bc) {
-    PFN_cuTensorMapEncodeTiled_v12000 encode = get_encode();
+    const auto encode = tensor_map_encoder();
     if (!encode) return false;
     const cuuint64_t gdim[3] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)planes};
     const cuuint64_t gstride[2] = {(cuuint64_t)W * 4, (cuuint64_t)H * W * 4};

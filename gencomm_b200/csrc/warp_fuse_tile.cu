@@ -27,16 +27,14 @@
 //
 // Requirements checked by the host: W % 4 == 0 and 16-byte aligned base (TMA global strides), at most
 // kTileMaxN agents per frame.  Otherwise gc_warp_fuse uses the gather kernels of warp_fuse.cu.
-#include <cuda.h>
-#include <cudaTypedefs.h>
 #include <stdlib.h>
 
-#include <type_traits>
-#include <utility>
-
+#include "ptx.cuh"
 #include "warp_common.cuh"
 
 namespace gc {
+
+using namespace ptx;
 
 constexpr int kTileMaxN = 5;
 constexpr int kMaxStages = 4;
@@ -69,59 +67,6 @@ struct TileCfg {
     static_assert(kThreads <= 1024, "block too large");
     static_assert((P & (P - 1)) == 0, "P must be a power of two");
 };
-
-// ---- PTX wrappers -----------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "WAIT_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra DONE_%=;\n\t"
-        "bra WAIT_%=;\n\t"
-        "DONE_%=:\n\t"
-        "}" ::"r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void tma_load_box(uint32_t dst, const CUtensorMap *map, int x, int y, int plane, uint32_t bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(x), "r"(y), "r"(plane), "r"(bar)
-        : "memory");
-}
-template <int kCount>
-__device__ __forceinline__ void consumer_sync() {   // named barrier 1: consumer warps only
-    asm volatile("bar.sync 1, %0;" ::"n"(kCount) : "memory");
-}
-// shared-memory accesses by 32-bit shared address + compile-time byte offset (folds into the LDS/STS immediate)
-template <int OFF>
-__device__ __forceinline__ float lds(uint32_t addr) {
-    float v;
-    asm volatile("ld.shared.f32 %0, [%1+%2];" : "=f"(v) : "r"(addr), "n"(OFF));
-    return v;
-}
-template <int OFF>
-__device__ __forceinline__ void sts(uint32_t addr, float v) {
-    asm volatile("st.shared.f32 [%0+%1], %2;" ::"r"(addr), "n"(OFF), "f"(v) : "memory");
-}
-template <int... Is, class F>
-__device__ __forceinline__ void static_for_impl(std::integer_sequence<int, Is...>, F &&f) {
-    (f(std::integral_constant<int, Is>{}), ...);
-}
-template <int N, class F>
-__device__ __forceinline__ void static_for(F &&f) {
-    static_for_impl(std::make_integer_sequence<int, N>{}, static_cast<F &&>(f));
-}
 
 struct TapS {
     float w_nw, w_ne, w_sw, w_se;
@@ -452,7 +397,7 @@ k_fuse_tile(const __grid_constant__ CUtensorMap tmap_box, const __grid_constant_
     else if (tid < TW + TH) s_ys[tid - TW] = base_coord(min(h0 + tid - TW, H - 1), H);
     if (tid == 0) {
         for (int s = 0; s < kMaxStages; ++s) { mbar_init(full_addr + 8u * s, 1); mbar_init(empty_addr + 8u * s, kConsumers / 32); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
         s_ident = 0xFFFFFFFFu;
     }
     __syncthreads();
@@ -624,23 +569,8 @@ k_fuse_tile(const __grid_constant__ CUtensorMap tmap_box, const __grid_constant_
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-static PFN_cuTensorMapEncodeTiled_v12000 get_encode() {
-    static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-            q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(p);
-        (void)cudaGetLastError();
-    }
-    return fn;
-}
-
 static bool encode_map(CUtensorMap *map, const float *feat, int W, int H, long long planes, int bw, int bh, int bc) {
-    PFN_cuTensorMapEncodeTiled_v12000 encode = get_encode();
+    const auto encode = tensor_map_encoder();
     if (!encode) return false;
     const cuuint64_t gdim[3] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)planes};
     const cuuint64_t gstride[2] = {(cuuint64_t)W * 4, (cuuint64_t)H * W * 4};

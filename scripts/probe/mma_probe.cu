@@ -3,8 +3,8 @@
 #include <cstdio>
 #include <cstdint>
 #include <cuda_runtime.h>
-#include "../../gencomm_b200/csrc/umma.cuh"
-using namespace gc::umma;
+#include "../../gencomm_b200/csrc/ptx.cuh"
+using namespace gc::ptx;
 
 __device__ __forceinline__ uint64_t desc(uint32_t saddr, uint32_t lbo, uint32_t sbo, uint32_t layout) {
     return make_desc(saddr, lbo, sbo) | ((uint64_t)layout << 61);
