@@ -63,6 +63,9 @@ SIGNATURES = {
                                   c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "gc_unet_forward": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
                                 c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "gc_unet_trace_floats": (c_size_t, [c_int, c_int, c_int]),
+    "gc_unet_trace": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
+                              c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "gc_me_param_floats": (c_size_t, []),
     "gc_me_packed_bytes": (c_size_t, [c_int]),
     "gc_me_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int]),

@@ -446,11 +446,22 @@ struct HostTail {     // trailing part of the host weight blob, after T * kC8Lay
     float norm_out_gamma[8], norm_out_beta[8];
 };
 
-// One DiffusionUNet evaluation; the result goes through k_conv_out's epilogue.
+// Tensor k of the layer trace of gc_unet_trace: hs0 (k = 0) or the output of middle layer k - 1, [A][h][w][8]; layers
+// 4 .. 18 (k = 5 .. 19) are half resolution.
+static size_t trace_offset(int k, int A, int H, int W) {
+    const int half = k < 5 ? 0 : (k > 20 ? 15 : k - 5);
+    return (size_t)A * ((size_t)(k - half) * H * W * 8 + (size_t)half * (H / 2) * (W / 2) * 8);
+}
+static void trace_copy(cudaStream_t st, const Act &a, int k, int A, int H, int W, float *trace) {
+    cudaMemcpyAsync(trace + trace_offset(k, A, H, W), a.data, (size_t)A * a.H * a.W * 8 * 4, cudaMemcpyDeviceToDevice, st);
+}
+
+// One DiffusionUNet evaluation; the result goes through k_conv_out's epilogue.  trace (gc_unet_trace, else NULL): every
+// layer's output is also written there.
 static int unet_eval(cudaStream_t st, int A, int C, int H, int W, const float *cond, UnetWorkspace &ws,
                      const C8Params *prm, const HostTail &tail, const float *w_in, const float *w_out,
                      const float *b_out, int mode, float c1, float c2, float sigma, const float *noise, float *pred,
-                     int precision, const float *rec_dev) {
+                     int precision, const float *rec_dev, float *trace = nullptr) {
     Act *p = ws.p, *q = ws.q;
     g_precision = precision;
     // cluster-resident middle (denoiser_cluster.cu): conv_in -> ONE launch for the 26 width-8 layers -> conv_out
@@ -465,10 +476,14 @@ static int unet_eval(cudaStream_t st, int A, int C, int H, int W, const float *c
             p[0].tiles = conv_in_tc_tiles(H, W);
             if (int rc = conv_in_tc(st, A, cond, ws.x, ws.tc_packed, bi, C, H, W, p[0].data, p[0].stats)) return rc;
         }
-        if (int rc = unet_middle_cluster(st, A, p[0].data, rec_dev, p[11].data, p[11].stats)) return rc;
+        if (int rc = unet_middle_cluster(st, A, p[0].data, rec_dev, p[11].data, p[11].stats, trace)) return rc;
         p[11].tiles = kCl;
         Affine8 aff;
         for (int i = 0; i < 8; ++i) { aff.gamma[i] = tail.norm_out_gamma[i]; aff.beta[i] = tail.norm_out_beta[i]; }
+        if (trace) {   // hs0 and the last layer's output are in p[0] / p[11]; the kernel wrote the others
+            trace_copy(st, p[0], 0, A, H, W, trace);
+            trace_copy(st, p[11], kC8Layers, A, H, W, trace);
+        }
         return conv_out_tc(st, A, p[11].data, p[11].stats, p[11].tiles, ws.tc_packed, b_out, aff, C, H, W, mode, c1, c2, sigma,
                            noise, ws.x, pred, 0);
     }
@@ -498,6 +513,9 @@ static int unet_eval(cudaStream_t st, int A, int C, int H, int W, const float *c
     resblock16(st, A, p[5], p[4], p[6], p[7], prm + 20);                                           // up.0.block.0  (pops hs[2])
     resblock16(st, A, p[7], p[2], p[8], p[9], prm + 22);                                           // up.0.block.1  (pops hs[1])
     resblock16(st, A, p[9], p[0], p[10], p[11], prm + 24);                                         // up.0.block.2  (pops hs[0])
+    if (trace) {   // tensor k: p[0 .. 4] = hs0, layers 0 .. 3; q[0 .. 14] = layers 4 .. 18; p[5 .. 11] = layers 19 .. 25
+        for (int k = 0; k <= kC8Layers; ++k) trace_copy(st, k < 5 ? p[k] : (k < 20 ? q[k - 5] : p[k - 15]), k, A, H, W, trace);
+    }
     Affine8 aff;
     for (int i = 0; i < 8; ++i) { aff.gamma[i] = tail.norm_out_gamma[i]; aff.beta[i] = tail.norm_out_beta[i]; }
     if ((precision & GC_PREC_TC_CONV_OUT) && conv_out_tc_eligible(C, H, W)) {
@@ -541,13 +559,17 @@ static int check_unet_args(int A, int C, int H, int W, int T) {
     return GC_OK;
 }
 
-// One denoiser evaluation x0 = UNet(cat[cond, x], t) for tests/diagnostics: writes pred [A][C][H][W].
-extern "C" int gc_unet_forward(const float *cond, const float *x, int total_agents, int t_index, const float *w_host,
-                               const float *w_dev, const float *w_cluster_dev, int C, int H, int W, int T, int precision,
-                               void *workspace, float *pred, void *stream) {
+extern "C" size_t gc_unet_trace_floats(int total_agents, int H, int W) {
+    if (total_agents <= 0 || H <= 0 || W <= 0) return 0;
+    return trace_offset(kC8Layers + 1, total_agents, H, W);
+}
+
+static int unet_forward(const char *name, const float *cond, const float *x, int total_agents, int t_index,
+                        const float *w_host, const float *w_dev, const float *w_cluster_dev, int C, int H, int W, int T,
+                        int precision, void *workspace, float *pred, float *trace, void *stream) {
     if (int rc = check_unet_args(total_agents, C, H, W, T)) return rc;
-    GC_REQUIRE(cond && x && w_host && w_dev && workspace && pred, GC_EINVAL, "gc_unet_forward: null pointer");
-    GC_REQUIRE(t_index >= 0 && t_index < T, GC_EINVAL, "gc_unet_forward: bad timestep");
+    GC_REQUIRE(cond && x && w_host && w_dev && workspace && pred, GC_EINVAL, "%s: null pointer", name);
+    GC_REQUIRE(t_index >= 0 && t_index < T, GC_EINVAL, "%s: bad timestep", name);
     cudaStream_t st = (cudaStream_t)stream;
     UnetWorkspace ws = carve_unet(workspace, total_agents, C, H, W);
     cudaMemcpyAsync(ws.x, x, (size_t)total_agents * C * H * W * 4, cudaMemcpyDeviceToDevice, st);
@@ -557,7 +579,24 @@ extern "C" int gc_unet_forward(const float *cond, const float *x, int total_agen
     if (precision & GC_PREC_BF16_TC)
         if (int rc = conv_tc_pack_weights(st, w_in, w_out, C, ws.tc_packed)) return rc;
     return unet_eval(st, total_agents, C, H, W, cond, ws, prm, tail, w_in, w_out, b_out, 0, 0.f, 0.f, 0.f, nullptr, pred,
-                     precision, w_cluster_dev ? w_cluster_dev + (size_t)t_index * kClLayers * kClRecFloats : nullptr);
+                     precision, w_cluster_dev ? w_cluster_dev + (size_t)t_index * kClLayers * kClRecFloats : nullptr, trace);
+}
+
+// One denoiser evaluation x0 = UNet(cat[cond, x], t) for tests/diagnostics: writes pred [A][C][H][W].
+extern "C" int gc_unet_forward(const float *cond, const float *x, int total_agents, int t_index, const float *w_host,
+                               const float *w_dev, const float *w_cluster_dev, int C, int H, int W, int T, int precision,
+                               void *workspace, float *pred, void *stream) {
+    return unet_forward("gc_unet_forward", cond, x, total_agents, t_index, w_host, w_dev, w_cluster_dev, C, H, W, T, precision,
+                        workspace, pred, nullptr, stream);
+}
+
+// gc_unet_forward that also writes hs0 and every middle layer's output to trace (include/gencomm_b200.h).
+extern "C" int gc_unet_trace(const float *cond, const float *x, int total_agents, int t_index, const float *w_host,
+                             const float *w_dev, const float *w_cluster_dev, int C, int H, int W, int T, int precision,
+                             void *workspace, float *pred, float *trace, void *stream) {
+    GC_REQUIRE(trace, GC_EINVAL, "gc_unet_trace: null pointer");
+    return unet_forward("gc_unet_trace", cond, x, total_agents, t_index, w_host, w_dev, w_cluster_dev, C, H, W, T, precision,
+                        workspace, pred, trace, stream);
 }
 
 extern "C" int gc_gencomm_sample(const float *feat, const float *cond, const int32_t *agent_offsets, int n_frames,

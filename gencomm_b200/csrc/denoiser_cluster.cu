@@ -469,7 +469,7 @@ __device__ __forceinline__ void epilogue_layer(Ctx &c, const LayerCfg &L, uint32
         const float4 o0 = make_float4(a[0], a[1], a[2], a[3]), o1 = make_float4(a[4], a[5], a[6], a[7]);
         sts4(out_base + poff, o0);
         sts4(out_base + poff + PXW * 16u, o1);
-        if (gout != nullptr) {   // last layer of the unfused variant: the raw tensor also goes to global memory (NHWC8)
+        if (gout != nullptr) {   // last layer (or every layer of the dump variant): the raw tensor also goes to global memory (NHWC8)
             float4 *dst = reinterpret_cast<float4 *>(gout + ((size_t)(y0 + r0) * PXW + px) * 8);
             dst[0] = o0;
             dst[1] = o1;
@@ -484,7 +484,8 @@ __device__ __forceinline__ void epilogue_layer(Ctx &c, const LayerCfg &L, uint32
 }
 
 // down.0.downsample (unet.py:59-78): pad (0,1,0,1) + 3x3 stride 2, no GroupNorm, on CUDA cores (thread = output pixel).
-__device__ __forceinline__ void down_layer(Ctx &c, const LayerCfg &L, uint32_t rec_saddr, float (&q8)[8]) {
+template <bool DUMP>
+__device__ __forceinline__ void down_layer(Ctx &c, const LayerCfg &L, uint32_t rec_saddr, float *gout, float (&q8)[8]) {
     const bool act = c.tid < 256;                      // 4 rows x 64 output pixels; the other warps only join the reduction
     if (!act) return;
     const int r = (c.tid >> 6) & 3, ox = c.tid & 63;
@@ -522,6 +523,11 @@ __device__ __forceinline__ void down_layer(Ctx &c, const LayerCfg &L, uint32_t r
     const uint32_t poff = (uint32_t)((r * 2) * 64 + ox) * 16u, out_base = c.smem + kOffF + buf_off(L.out);
     sts4(out_base + poff, make_float4(acc[0], acc[1], acc[2], acc[3]));
     sts4(out_base + poff + 64u * 16u, make_float4(acc[4], acc[5], acc[6], acc[7]));
+    if (DUMP) {   // layer dump (gc_unet_trace): NHWC8 [32][64][8] of this agent
+        float4 *dst = reinterpret_cast<float4 *>(gout + ((size_t)((int)c.rank * 4 + r) * 64 + ox) * 8);
+        dst[0] = make_float4(acc[0], acc[1], acc[2], acc[3]);
+        dst[1] = make_float4(acc[4], acc[5], acc[6], acc[7]);
+    }
 #pragma unroll
     for (int p = 0; p < 4; ++p) {
         q8[2 * p] = acc[2 * p] + acc[2 * p + 1];
@@ -529,9 +535,19 @@ __device__ __forceinline__ void down_layer(Ctx &c, const LayerCfg &L, uint32_t r
     }
 }
 
+// Global-memory offset (floats) of tensor k of the layer dump of gc_unet_trace at 64 x 128: tensor 0 = hs0, tensor 1 + l =
+// the output of layer l, each [A][h][w][8]; tensors 5 .. 19 (layers 4 .. 18) are half resolution.
+__device__ __forceinline__ size_t dump_offset(int k, int n_agents) {
+    const int half = k < 5 ? 0 : (k > 20 ? 15 : k - 5);
+    return (size_t)n_agents * ((size_t)(k - half) * (64 * 128 * 8) + (size_t)half * (32 * 64 * 8));
+}
+
 // The 26 middle layers of one UNet evaluation.  rec_g: this step's layer records in global memory.  On entry the input
-// tensor (F0) and its statistics have been pushed (hand-over c.sync_n - 1 is in flight).
-__device__ __forceinline__ void middle_layers(Ctx &c, const float *rec_g, float *gout, float *gstats) {
+// tensor (F0) and its statistics have been pushed (hand-over c.sync_n - 1 is in flight).  DUMP: every layer's output also
+// goes to `dump` (the layout of dump_offset) except the last one's, which goes to gout as in the production variant.
+template <bool DUMP>
+__device__ __forceinline__ void middle_layers(Ctx &c, const float *rec_g, float *gout, float *gstats, float *dump, int agent,
+                                              int n_agents) {
     if (c.tid == 32) {   // records 0 and 1; record l + 2 follows at the end of layer l (a full layer ahead of its use)
         bulk_load(c.smem + kOffRec, rec_g, kClRecBytes, MISC_ADDR(c, rec_bar));
         bulk_load(c.smem + kOffRec + kClRecBytes, rec_g + kClRecFloats, kClRecBytes, MISC_ADDR(c, rec_bar) + 8u);
@@ -569,15 +585,18 @@ __device__ __forceinline__ void middle_layers(Ctx &c, const float *rec_g, float 
 #pragma unroll
         for (int i = 0; i < 8; ++i) q8[i] = 0.0f;
         const bool last = l == kClLayers - 1;
+        float *lout = nullptr;
+        if (DUMP && !last)
+            lout = dump + dump_offset(l + 1, n_agents) + (size_t)agent * (L.half ? 32 * 64 * 8 : 64 * 128 * 8);
         if (L.kind == kDownK) {
-            down_layer(c, L, rec_saddr, q8);
+            down_layer<DUMP>(c, L, rec_saddr, lout, q8);
         } else {
             if (L.kind == kUpK) stage_layer<1, false, true, false>(c, L);
             else if (L.half) { if (L.cin == 8) stage_layer<1, true, false, true>(c, L); else stage_layer<2, true, false, true>(c, L); }
             else { if (L.cin == 8) stage_layer<1, false, false, true>(c, L); else stage_layer<2, false, false, true>(c, L); }
             GC_TRACE(c, 4);
-            if (L.half) epilogue_layer<true>(c, L, rec_saddr, nullptr, q8);
-            else epilogue_layer<false>(c, L, rec_saddr, last ? gout : nullptr, q8);
+            if (L.half) epilogue_layer<true>(c, L, rec_saddr, DUMP ? lout : nullptr, q8);
+            else epilogue_layer<false>(c, L, rec_saddr, last ? gout : (DUMP ? lout : nullptr), q8);
         }
         GC_TRACE(c, 12);
         push_stats(c, q8, L.out, last ? gstats : nullptr);
@@ -592,10 +611,13 @@ __device__ __forceinline__ void middle_layers(Ctx &c, const float *rec_g, float 
 // ------------------------------------------------------------------------------------------------
 // Unfused variant: h0 = conv_in output (NHWC8, global) -> 26 layers -> input of norm_out (NHWC8, global) + its
 // per-band GroupNorm partial sums [A][8 bands][8] for k_conv_out_tc.  One cluster per agent (grid-stride).
+// DUMP (gc_unet_trace only): layers 0 .. 24 are also stored to layer_dump (see dump_offset); the production variant is
+// DUMP = false and never reads the pointer.
 // ------------------------------------------------------------------------------------------------
+template <bool DUMP>
 __global__ void __cluster_dims__(kCl, 1, 1) __launch_bounds__(kThreads, 1)
 k_unet_middle_cluster(const float *__restrict__ h0, const float *__restrict__ rec_g, float *__restrict__ out,
-                      float *__restrict__ stats_out, int n_agents, int dbg, long long *trace) {
+                      float *__restrict__ stats_out, int n_agents, int dbg, long long *trace, float *__restrict__ layer_dump) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     Ctx c;
     c.smem = smem_u32(smem_raw);
@@ -665,7 +687,8 @@ k_unet_middle_cluster(const float *__restrict__ h0, const float *__restrict__ re
         } else {
             ++c.sync_n;
         }
-        middle_layers(c, rec_g, out + (size_t)agent * 64 * 128 * 8, stats_out + (size_t)agent * kCl * 8);
+        middle_layers<DUMP>(c, rec_g, out + (size_t)agent * 64 * 128 * 8, stats_out + (size_t)agent * kCl * 8, layer_dump, agent,
+                            n_agents);
         // the hand-over of layer 25 must be consumed before the next agent's F0 load: a neighbour reads this CTA's F0 / F2
         // rows until it has finished layer 24 / 25
         // (every hand-over is waited for exactly once: this is the wait of layer 25's)
@@ -688,7 +711,10 @@ bool unet_cluster_eligible(int C, int H, int W) {
     return H == 64 && W == 128;
 }
 
-static int cluster_grid(const void *kernel, size_t smem, int n_agents, int *n_clusters) {
+// one cache (and one shared-memory attribute) per kernel instantiation
+template <bool DUMP>
+static int cluster_grid(size_t smem, int n_agents, int *n_clusters) {
+    const void *kernel = (const void *)cl::k_unet_middle_cluster<DUMP>;
     static int cached = -1;
     if (cached < 0) {
         cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -710,9 +736,11 @@ static int cluster_grid(const void *kernel, size_t smem, int n_agents, int *n_cl
     return GC_OK;
 }
 
-int unet_middle_cluster(cudaStream_t st, int A, const float *h0, const float *rec_dev, float *out, float *stats_out) {
+int unet_middle_cluster(cudaStream_t st, int A, const float *h0, const float *rec_dev, float *out, float *stats_out,
+                        float *layer_dump) {
     int n_clusters = 0;
-    if (int rc = cluster_grid((const void *)cl::k_unet_middle_cluster, cl::kSmemBytes, A, &n_clusters)) return rc;
+    if (int rc = layer_dump ? cluster_grid<true>(cl::kSmemBytes, A, &n_clusters) : cluster_grid<false>(cl::kSmemBytes, A, &n_clusters))
+        return rc;
     static int dbg = -1;
     if (dbg < 0) { const char *e = getenv("GC_CL_DEBUG"); dbg = e ? atoi(e) : 0; }
     static long long *trace = nullptr;
@@ -720,7 +748,12 @@ int unet_middle_cluster(cudaStream_t st, int A, const float *h0, const float *re
         cudaMalloc(&trace, 2 * kClLayers * 16 * sizeof(long long));
         cudaMemset(trace, 0, 2 * kClLayers * 16 * sizeof(long long));
     }
-    cl::k_unet_middle_cluster<<<n_clusters * kCl, cl::kThreads, cl::kSmemBytes, st>>>(h0, rec_dev, out, stats_out, A, dbg, trace);
+    if (layer_dump)
+        cl::k_unet_middle_cluster<true><<<n_clusters * kCl, cl::kThreads, cl::kSmemBytes, st>>>(h0, rec_dev, out, stats_out, A, dbg,
+                                                                                                trace, layer_dump);
+    else
+        cl::k_unet_middle_cluster<false><<<n_clusters * kCl, cl::kThreads, cl::kSmemBytes, st>>>(h0, rec_dev, out, stats_out, A, dbg,
+                                                                                                 trace, nullptr);
     if (trace != nullptr) {   // debug only: dump the timeline of the last agent CTA 0 processed
         cudaStreamSynchronize(st);
         long long h[2 * kClLayers * 16];

@@ -20,7 +20,9 @@ bool unet_cluster_eligible(int C, int H, int W);
 
 // 26 middle layers: h0 [A][64][128][8] (conv_in output, NHWC8) -> out [A][64][128][8] (input of norm_out) +
 // stats_out [A][8][8] (GroupNorm partial sums per row band, the format k_conv_out_tc consumes with tiles = 8).
-// rec_dev: kClLayers records of the step being evaluated.
-int unet_middle_cluster(cudaStream_t st, int A, const float *h0, const float *rec_dev, float *out, float *stats_out);
+// rec_dev: kClLayers records of the step being evaluated.  layer_dump (gc_unet_trace, else NULL): the outputs of layers
+// 0 .. 24 are also written there, in the layout of the trace of include/gencomm_b200.h (tensor 1 + l at its offset).
+int unet_middle_cluster(cudaStream_t st, int A, const float *h0, const float *rec_dev, float *out, float *stats_out,
+                        float *layer_dump);
 
 }  // namespace gc

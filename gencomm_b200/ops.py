@@ -326,6 +326,38 @@ def unet_forward(cond, x, t_index, w_host, w_dev, T, workspace=None, precision=0
     return pred
 
 
+def unet_trace(cond, x, t_index, w_host, w_dev, T, workspace=None, precision=0, w_cluster=None, pred=None, trace=None):
+    """unet_forward that also returns the activations: (pred, [27 NHWC8 tensors]) with tensor 0 = conv_in output and
+    tensor 1 + l = the output of middle layer l ([A, H/2, W/2, 8] for l = 4 .. 18, [A, H, W, 8] otherwise).
+    pred / trace may be passed in (trace: a flat float32 tensor of gc_unet_trace_floats(A, H, W) elements)."""
+    lib = _lib.load()
+    _chk(cond, "cond", torch.float32, 4)
+    _chk(x, "x", torch.float32, 4)
+    _chk(w_dev, "w_dev", torch.float32, 1)
+    A, C, H, W = x.shape
+    if tuple(cond.shape) != (A, 2, H, W):
+        raise ValueError("cond must be [A,2,H,W]")
+    _check_blobs(lib, w_host, w_dev, C, T)
+    if workspace is None:
+        workspace = torch.empty(lib.gc_gencomm_workspace_bytes(A, C, H, W), dtype=torch.uint8, device=x.device)
+    n = lib.gc_unet_trace_floats(A, H, W)
+    pred = torch.empty_like(x) if pred is None else pred
+    trace = torch.empty(n, dtype=torch.float32, device=x.device) if trace is None else trace
+    _chk(pred, "pred", torch.float32, 4)
+    _chk(trace, "trace", torch.float32, 1)
+    if pred.shape != x.shape or trace.numel() != n:
+        raise ValueError("unet_trace: pred must be like x and trace must hold gc_unet_trace_floats(A, H, W) floats")
+    _lib.check(lib.gc_unet_trace(_ptr(cond), _ptr(x), A, int(t_index), _host_ptr(w_host), _ptr(w_dev),
+                                 _cluster_ptr(lib, w_cluster, T), C, H, W, int(T), int(precision), _ptr(workspace),
+                                 _ptr(pred), _ptr(trace), _stream()), "gc_unet_trace")
+    tensors, off = [], 0
+    for k in range(27):
+        h, w = (H // 2, W // 2) if 5 <= k <= 19 else (H, W)
+        tensors.append(trace[off:off + A * h * w * 8].view(A, h, w, 8))
+        off += A * h * w * 8
+    return pred, tensors
+
+
 def gencomm_sample(feat, cond, agent_offsets, noise0, step_noise, w_host, w_dev, schedule, T, workspace=None, out=None,
                    precision=0, w_cluster=None):
     """GenComm eval sampler; feat [sumN,C,H,W], cond [sumN,2,H,W], noise0 like feat, step_noise [>=T-1,sumN,C,H,W]."""

@@ -208,6 +208,19 @@ int gc_unet_forward(const float *cond, const float *x, int total_agents, int t_i
                     const float *w_host /*[host]*/, const float *w_dev, const float *w_cluster_dev /* or NULL */, int C,
                     int H, int W, int T, int precision /* GC_PREC_* */, void *workspace, float *pred, void *stream);
 
+/* gc_unet_forward that also writes the activations of the evaluation to trace [device], for per-layer tests:
+ * gc_unet_trace_floats(total_agents, H, W) floats holding 27 NHWC8 fp32 tensors back to back,
+ *   tensor 0      hs0 = conv_in output                      [A][H][W][8]
+ *   tensor 1 + l  output of middle layer l (l = 0 .. 25, the execution order of the 26 width-8 convolutions:
+ *                 down.0.block.0 conv1, conv2, down.0.block.1 conv1, conv2, down.0.downsample, down.1.block.0 conv1, ...,
+ *                 up.0.block.2 conv2), [A][H/2][W/2][8] for l = 4 .. 18 (tensors 5 .. 19), [A][H][W][8] otherwise.
+ * pred is bit-identical to gc_unet_forward's for every precision. */
+size_t gc_unet_trace_floats(int total_agents, int H, int W);
+int gc_unet_trace(const float *cond, const float *x, int total_agents, int t_index,
+                  const float *w_host /*[host]*/, const float *w_dev, const float *w_cluster_dev /* or NULL */, int C,
+                  int H, int W, int T, int precision /* GC_PREC_* */, void *workspace, float *pred, float *trace,
+                  void *stream);
+
 /* ---------------------------------------------------------------------------------------------
  * (8f rank 1) MessageExtractorv2.forward (models/gencomm_modules/message_extractor_v2.py:114-120)
  *   = BEVDeformableExtractor.forward (:96-112): offset1 (3x3 conv C->18) -> torchvision DeformConv2d (3x3, C->64,
