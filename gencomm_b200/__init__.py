@@ -18,6 +18,8 @@ from .det_tail import DetectionHeads, DoubleConv, DownsampleConv  # noqa: F401
 from .backbone import BaseBEVBackbone  # noqa: F401
 from .postprocess import VoxelPostprocessor  # noqa: F401
 from .lss import VoxelPooling, gen_dx_bx, voxel_pooling  # noqa: F401
+from . import eval_utils  # noqa: F401
+from .eval_utils import DetectionEvaluator, caluclate_tp_fp  # noqa: F401
 
 from .heter_model_baseline_w_gencomm_stage1 import HeterModelBaselineWGenComm  # noqa: F401
 from .heter_model_baseline_w_gencomm_stage2 import HeterModelBaselineWDiffCommStage2  # noqa: F401

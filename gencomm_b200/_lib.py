@@ -104,6 +104,9 @@ SIGNATURES = {
     "gc_postprocess_workspace_bytes": (c_size_t, [c_int, c_int]),
     "gc_postprocess": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                                ctypes.POINTER(PostParams), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "gc_eval_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "gc_eval_match": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p, c_int,
+                              c_void_p, c_void_p, c_void_p, c_void_p]),
 }
 
 _lib = None

@@ -669,6 +669,51 @@ def postprocess(cls_preds, reg_preds, dir_preds, anchors, params, tfm=None, work
 
 
 # --------------------------------------------------------------------------------------------
+# evaluation: greedy detection -> ground-truth matching (eval_utils.caluclate_tp_fp)
+# --------------------------------------------------------------------------------------------
+EVAL_MAX_BOXES = 1024
+EVAL_MAX_THRESHOLDS = 8
+
+
+def eval_match(det_boxes, det_scores, det_counts, gt_boxes, gt_counts, thresholds, out=None):
+    """det_boxes [B,K,8,3] f32, det_scores [B,K] f32, det_counts [B] i32, gt_boxes [B,G,8,3] f32, gt_counts [B] i32 (cuda),
+    thresholds: 1..8 IoU thresholds -> (sorted_scores [B,K] f32, tp [B,T,K] u8).  Per frame and threshold the detections
+    are sorted by descending score (ties keep input order) and greedily matched, as eval_utils.caluclate_tp_fp does;
+    tp[b,t,i] = 1 for a true positive, 0 for a false positive or i >= det_counts[b].  ``out`` = (sorted_scores, tp) to
+    write into.  Asynchronous (counts stay on the device; values outside [0, K] / [0, G] are clamped)."""
+    lib = _lib.load()
+    _chk(det_boxes, "det_boxes", torch.float32, 4)
+    _chk(det_scores, "det_scores", torch.float32, 2)
+    _chk(det_counts, "det_counts", torch.int32, 1)
+    _chk(gt_boxes, "gt_boxes", torch.float32, 4)
+    _chk(gt_counts, "gt_counts", torch.int32, 1)
+    B, K = det_boxes.shape[:2]
+    G = gt_boxes.shape[1]
+    if tuple(det_boxes.shape[2:]) != (8, 3) or tuple(det_scores.shape) != (B, K) or tuple(det_counts.shape) != (B,):
+        raise ValueError("eval_match: det_boxes must be [B,K,8,3], det_scores [B,K] and det_counts [B]")
+    if tuple(gt_boxes.shape) != (B, G, 8, 3) or tuple(gt_counts.shape) != (B,):
+        raise ValueError("eval_match: gt_boxes must be [B,G,8,3] and gt_counts [B]")
+    if not (1 <= K <= EVAL_MAX_BOXES and 1 <= G <= EVAL_MAX_BOXES):
+        raise ValueError(f"eval_match: K and G must be in 1..{EVAL_MAX_BOXES}, got K={K}, G={G}")
+    th = np.ascontiguousarray(thresholds, dtype=np.float64).reshape(-1)
+    if not 1 <= th.size <= EVAL_MAX_THRESHOLDS:
+        raise ValueError(f"eval_match: 1..{EVAL_MAX_THRESHOLDS} thresholds, got {th.size}")
+    dev = det_boxes.device
+    workspace = torch.empty(lib.gc_eval_workspace_bytes(B, K, G), dtype=torch.uint8, device=dev)
+    if out is None:
+        out = (torch.empty(B, K, dtype=torch.float32, device=dev), torch.empty(B, th.size, K, dtype=torch.uint8, device=dev))
+    sorted_scores, tp = out
+    _chk(sorted_scores, "sorted_scores", torch.float32, 2)
+    _chk(tp, "tp", torch.uint8, 3)
+    if tuple(sorted_scores.shape) != (B, K) or tuple(tp.shape) != (B, th.size, K):
+        raise ValueError("eval_match: out must be (sorted_scores [B,K], tp [B,T,K])")
+    _lib.check(lib.gc_eval_match(_ptr(det_boxes), _ptr(det_scores), _ptr(det_counts), K, _ptr(gt_boxes), _ptr(gt_counts), G, B,
+                                 th.ctypes.data_as(ctypes.c_void_p), th.size, _ptr(workspace), _ptr(sorted_scores), _ptr(tp),
+                                 _stream()), "gc_eval_match")
+    return sorted_scores, tp
+
+
+# --------------------------------------------------------------------------------------------
 # (8f rank 4) LSS voxel pooling
 # --------------------------------------------------------------------------------------------
 def lss_voxel_pooling(geom_feats, x, dx, bx, nx, vector=True, deterministic=False):

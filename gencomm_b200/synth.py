@@ -269,3 +269,77 @@ def lss_frustum(seed, B=2, N=2, D=12, H=8, W=11, C=16, grid_conf=None, coarse_fr
     geom = torch.stack([xs, ys, zs], dim=-1).float()
     x = torch.randn(*shape, C, generator=g)
     return geom, x
+
+
+_CORNER_TEMPLATE = np.array([[1, -1, -1], [1, 1, -1], [-1, 1, -1], [-1, -1, -1],
+                             [1, -1, 1], [1, 1, 1], [-1, 1, 1], [-1, -1, 1]], dtype=np.float64) / 2
+
+
+def box_corners(boxes):
+    """[N,7] (x, y, z, l, w, h, yaw) -> [N,8,3] f32 corners in the order of box_utils.boxes_to_corners_3d (order 'lhw',
+    utils/box_utils.py:152-203): template (+-l/2, +-w/2, +-h/2), rotation by yaw about z, then the centre."""
+    b = np.asarray(boxes, dtype=np.float64).reshape(-1, 7)
+    c = b[:, None, 3:6] * _CORNER_TEMPLATE[None]
+    co, si = np.cos(b[:, 6])[:, None], np.sin(b[:, 6])[:, None]
+    x = c[..., 0] * co - c[..., 1] * si + b[:, None, 0]
+    y = c[..., 0] * si + c[..., 1] * co + b[:, None, 1]
+    return np.stack([x, y, c[..., 2] + b[:, None, 2]], axis=-1).astype(np.float32)
+
+
+def _cars(g, n):
+    """n car-sized boxes [n,7] (l 3.5-5, w 1.6-2.1, h 1.4-1.8 m, any yaw) with all corners inside the OPV2V-H gt_range."""
+    xmin, ymin, _, xmax, ymax, _ = OPV2V_H_RANGE
+    return np.stack([g.uniform(xmin + 3.5, xmax - 3.5, n), g.uniform(ymin + 3.5, ymax - 3.5, n), g.uniform(-1.9, -0.9, n),
+                     g.uniform(3.5, 5.0, n), g.uniform(1.6, 2.1, n), g.uniform(1.4, 1.8, n),
+                     g.uniform(-np.pi, np.pi, n)], axis=1)
+
+
+def _jitter(g, boxes, pos, size, yaw):
+    out = boxes.copy()
+    out[:, 0:2] += g.normal(0.0, pos, (len(boxes), 2))
+    out[:, 3:5] *= 1.0 + g.normal(0.0, size, (len(boxes), 2))
+    out[:, 6] += g.normal(0.0, yaw, len(boxes))
+    return out
+
+
+def eval_frames(seed, n_frames, k_max=1000, g_max=200, n_gt=(20, 200), no_det=(), no_gt=(), full=(), score_step=None):
+    """Padded detections and ground truths of ``n_frames`` frames for the evaluation matching (eval_utils.caluclate_tp_fp):
+
+        det_boxes [B,k_max,8,3] f32, det_scores [B,k_max] f32, det_counts [B] i32,
+        gt_boxes [B,g_max,8,3] f32, gt_counts [B] i32       (torch, host; rows beyond a count are zero)
+
+    Ground truths: n_gt[0]..n_gt[1] car-sized boxes (at most g_max) with random yaw inside the OPV2V-H range.  Detections,
+    in random order: a jittered copy of ~80 % of the ground truths, a second, looser copy of ~30 % of those (duplicates,
+    so the greedy order matters) and free false positives; scores U(0.2, 1), rounded to multiples of ``score_step`` if
+    given (many equal scores).  Frames listed in ``no_det`` have no detection, in ``no_gt`` no ground truth, and in
+    ``full`` exactly k_max detections."""
+    B = int(n_frames)
+    det = np.zeros((B, k_max, 8, 3), np.float32)
+    scores = np.zeros((B, k_max), np.float32)
+    gts = np.zeros((B, g_max, 8, 3), np.float32)
+    det_counts = np.zeros(B, np.int32)
+    gt_counts = np.zeros(B, np.int32)
+    for f in range(B):
+        g = np.random.default_rng(BASE_SEED + 1000 * int(seed) + 7919 * 11 + f)
+        n_g = 0 if f in no_gt else min(int(g.integers(n_gt[0], n_gt[1] + 1)), g_max)
+        gt = _cars(g, n_g)
+        hit = gt[g.random(n_g) < 0.8]
+        dup = hit[g.random(len(hit)) < 0.3]
+        parts = [_jitter(g, hit, 0.25, 0.06, 0.08), _jitter(g, dup, 0.6, 0.1, 0.2),
+                 _cars(g, int(g.integers(2, 10 + n_g // 5)))]
+        d = np.concatenate(parts)
+        if f in full and len(d) < k_max:
+            d = np.concatenate([d, _cars(g, k_max - len(d))])
+        d = d[g.permutation(len(d))][:k_max]
+        if f in no_det:
+            d = d[:0]
+        s = g.uniform(0.2, 1.0, len(d))
+        if score_step:
+            s = np.round(s / score_step) * score_step
+        gts[f, :n_g] = box_corners(gt)
+        det[f, :len(d)] = box_corners(d)
+        scores[f, :len(d)] = s.astype(np.float32)
+        det_counts[f], gt_counts[f] = len(d), n_g
+    return {"det_boxes": torch.from_numpy(det), "det_scores": torch.from_numpy(scores),
+            "det_counts": torch.from_numpy(det_counts), "gt_boxes": torch.from_numpy(gts),
+            "gt_counts": torch.from_numpy(gt_counts)}

@@ -353,6 +353,29 @@ int gc_lss_voxel_pooling_det(const float *geom_feats, const float *x, long long 
                              const float *dx /*[3] host*/, const float *bx /*[3] host*/, const int *nx /*[3] host*/,
                              void *workspace, float *out, void *stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Evaluation matching: eval_utils.caluclate_tp_fp (utils/eval_utils.py) with common_utils.convert_format / compute_iou
+ * (utils/common_utils.py:230-270), for n_frames frames and n_thresh IoU thresholds in one call.  Per frame and threshold:
+ * sort the detections by descending score, then greedily, in that order, match each to the still-unmatched ground truth
+ * of largest IoU; it is a TP when that IoU (float32, widened to double) is >= the threshold, else a FP.
+ *   det_boxes [B][k_max][8][3], det_scores [B][k_max], det_counts [B] (gc_postprocess's outputs), gt_boxes [B][g_max][8][3],
+ *   gt_counts [B]; polygons are the bottom-face corners 0..3 (x, y) in float64, IoU = inter / (|A| + |B| - inter) as
+ *   float32 (the float64 convex clipping of gc_postprocess's NMS; shapely parity unpinned).
+ *   -> sorted_scores [B][k_max] f32 (descending; 0 beyond the count), tp [B][n_thresh][k_max] u8 (1 = TP; FP = 1 - tp
+ *   below the count, 0 beyond it).
+ *   Ties: equal scores keep their input order (the reference's np.argsort(-score) leaves them unspecified); equal IoUs
+ *   match the lowest ground-truth index (np.argmax); a NaN IoU (zero-area detection against a zero-area ground truth)
+ *   makes the detection a TP matched to the first NaN, as numpy's max / argmax do.  Scores must be finite.
+ *   Device counts outside [0, k_max] / [0, g_max] are clamped into that range.
+ *   Argument errors (GC_EINVAL): NULL pointers, n_frames outside 1..65535, k_max or g_max outside 1..1024, n_thresh
+ *   outside 1..8.  workspace: gc_eval_workspace_bytes bytes (0 for arguments outside those ranges).  No allocation, no
+ *   host synchronisation.
+ * ------------------------------------------------------------------------------------------- */
+size_t gc_eval_workspace_bytes(int n_frames, int k_max, int g_max);
+int gc_eval_match(const float *det_boxes, const float *det_scores, const int *det_counts, int k_max, const float *gt_boxes,
+                  const int *gt_counts, int g_max, int n_frames, const double *iou_thresh /*[n_thresh] host*/, int n_thresh,
+                  void *workspace, float *sorted_scores, uint8_t *tp, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
