@@ -21,6 +21,7 @@ from .lss import VoxelPooling, gen_dx_bx, voxel_pooling  # noqa: F401
 from . import eval_utils  # noqa: F401
 from .eval_utils import DetectionEvaluator, caluclate_tp_fp  # noqa: F401
 
+from .heter_model_baseline import HeterModelBaseline  # noqa: F401
 from .heter_model_baseline_w_gencomm_stage1 import HeterModelBaselineWGenComm  # noqa: F401
 from .heter_model_baseline_w_gencomm_stage2 import HeterModelBaselineWDiffCommStage2  # noqa: F401
 
@@ -33,7 +34,8 @@ def create_model(hypes):
     try:
         lib = importlib.import_module(f"{__name__}.{name}")
     except ModuleNotFoundError as e:
-        raise NotImplementedError(f"gencomm_b200 has no model {name!r} (GenComm stage 1 / stage 2 detectors only)") from e
+        raise NotImplementedError(f"gencomm_b200 has no model {name!r} (HeterModelBaseline and the GenComm stage 1 / "
+                                  "stage 2 detectors only)") from e
     target = name.replace('_', '').lower()
     for attr, cls in lib.__dict__.items():
         if attr.lower() == target:

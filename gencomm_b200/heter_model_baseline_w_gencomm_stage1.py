@@ -26,142 +26,39 @@ re-assembly of the modalities (:215-228) -- runs here.  The other fusion network
 Extensions (ignored by the reference): ``data_dict['inputs_m{k}']`` may carry raw ``points`` + ``point_offsets`` (see
 ``modules.PointPillar``); ``data_dict['gencomm_noise'] = (noise0, step_noises)`` injects pre-drawn sampler noise
 (parity tests).
+
+The encoder / backbone / shrink header branches, the camera zero-padding, the per-agent re-assembly, the fusion and the
+heads are ``HeterModelBaseline``'s (``heter_model_baseline.py``, the same detector without GenComm); this class adds the
+message extractors, the sampler and the Enhancer.
 """
-from collections import Counter, OrderedDict
-
-import os
-
 import torch
-import torch.nn as nn
 
-from .backbone import BaseBEVBackbone
-from .det_tail import DetectionHeads, DownsampleConv
 from .enhancer import Enhancer
 from .gencomm import GenComm
+from .heter_model_baseline import HeterModelBaseline
 from .message_extractor import MessageExtractorv2
-from .modules import AttFusion, BEVFeatureInput, MaxFusion, PointPillar, center_crop, normalize_pairwise_tfm
-
-_ENCODERS = {("lidar", "pointpillar"): PointPillar, ("camera", "liftsplatshoot"): BEVFeatureInput}
+from .modules import normalize_pairwise_tfm
 
 
-class _HeadsMixin:
-    """The three 1x1 heads keep their reference names / state_dict keys; they are evaluated as one GEMM."""
-
-    def _run_heads(self, x, suffix=""):
-        key = "_heads" + suffix
-        heads = getattr(self, key, None)
-        if heads is None:
-            heads = DetectionHeads.__new__(DetectionHeads)
-            nn.Module.__init__(heads)
-            heads.cls_head = getattr(self, "cls_head" + suffix)
-            heads.reg_head = getattr(self, "reg_head" + suffix)
-            heads.dir_head = getattr(self, "dir_head" + suffix)
-            heads._key, heads._blobs = None, None
-            object.__setattr__(self, key, heads)     # not registered: the convs stay owned by this module
-        return heads(x)
-
-
-class HeterModelBaselineWGenComm(_HeadsMixin, nn.Module):
+class HeterModelBaselineWGenComm(HeterModelBaseline):
     GENCOMM_KEY = "gencomm"            # stage 2 reads args['diffcomm'] (…_stage2.py:36)
     MISSING_KEEP = 0.4                 # mask = rand > 0.4 (…_stage1.py:233)
     CROP_MESSAGE = False               # stage 2 pads the camera agents' messages too (…_stage2.py:236); stage 1 does not
 
-    def __init__(self, args):
-        super().__init__()
-        self.args = args
+    def _add_sampler(self, args):
         self.gencomm = GenComm(args[self.GENCOMM_KEY])
         self.missing_message = args.get('missing_message', False)
-        self.modality_name_list = [x for x in args.keys() if x.startswith("m") and x[1:].isdigit()]
-        self.ego_modality = args['ego_modality']
-        self.cav_range = args['lidar_range']
-        self.sensor_type_dict = OrderedDict()
 
-        for modality_name in self.modality_name_list:
-            setting = args[modality_name]
-            self.sensor_type_dict[modality_name] = setting['sensor_type']
-            target = setting['core_method'].replace('_', '').lower()
-            if (setting['sensor_type'], target) not in _ENCODERS:
-                raise NotImplementedError(
-                    f"gencomm_b200: modality {modality_name} ({setting['sensor_type']}/{setting['core_method']}) -- LiDAR "
-                    "point_pillar encoders and camera lift_splat_shoot BEV features are on the B200 hot path")
-            setattr(self, f"encoder_{modality_name}", _ENCODERS[(setting['sensor_type'], target)](setting['encoder_args']))
-            if setting['sensor_type'] == 'camera':      # …_stage1.py:88-92
-                grid = setting['camera_mask_args']['grid_conf']
-                setattr(self, f"crop_ratio_W_{modality_name}", self.cav_range[3] / grid['xbound'][1])
-                setattr(self, f"crop_ratio_H_{modality_name}", self.cav_range[4] / grid['ybound'][1])
-            setattr(self, f"depth_supervision_{modality_name}", False)
-            if setting['backbone_args'] == 'identity':
-                setattr(self, f"backbone_{modality_name}", nn.Identity())
-            else:
-                setattr(self, f"backbone_{modality_name}",
-                        BaseBEVBackbone(setting['backbone_args'], setting['backbone_args'].get('inplanes', 64)))
-            setattr(self, f"shrinker_{modality_name}", DownsampleConv(setting['shrink_header']))
-            setattr(self, f"message_extractor_{modality_name}", self._make_message_extractor(args))
+    def _add_message_extractor(self, modality_name, args):
+        setattr(self, f"message_extractor_{modality_name}", self._make_message_extractor(args))
 
-        # metric extents for the pose normalisation (…_stage1.py:94-97)
-        self.H = self.cav_range[4] - self.cav_range[1]
-        self.W = self.cav_range[3] - self.cav_range[0]
-        self.fake_voxel_size = 1
-        self.gmatch = bool(args.get('gmatch', False))
-        self.num_class = args['num_class'] if "num_class" in args else 1
-        anchors, bins = args['anchor_number'], args['dir_args']['num_bins']
-
-        self.supervise_single = bool(args.get("supervise_single", False))
-        if self.supervise_single:
-            c = args['in_head_single']
-            self.cls_head_single = nn.Conv2d(c, anchors * self.num_class * self.num_class, kernel_size=1)
-            self.reg_head_single = nn.Conv2d(c, anchors * 7 * self.num_class, kernel_size=1)
-            self.dir_head_single = nn.Conv2d(c, anchors * bins, kernel_size=1)
-
-        if args['fusion_method'] == "max":
-            self.fusion_net = MaxFusion()
-        elif args['fusion_method'] == "att":
-            self.fusion_net = AttFusion(args['att']['feat_dim'])
-        else:
-            raise NotImplementedError(f"gencomm_b200: fusion_method {args['fusion_method']!r} -- max and att are on the "
-                                      "B200 hot path (SURVEY.md 8a rows a8/a9)")
-
-        self.shrink_flag = 'shrink_header' in args
-        if self.shrink_flag:
-            self.shrink_conv = DownsampleConv(args['shrink_header'])
-
-        self.cls_head = nn.Conv2d(args['in_head'], anchors * self.num_class * self.num_class, kernel_size=1)
-        self.reg_head = nn.Conv2d(args['in_head'], 7 * anchors * self.num_class, kernel_size=1)
-        self.dir_head = nn.Conv2d(args['in_head'], bins * anchors, kernel_size=1)
-
+    def _add_enhancer(self, args):
         if 'enhancer' in args:
             self.enhancer = Enhancer(args['enhancer']['in_ch'], [8, 8], 4)
-
-        self.compress = False
-        if 'compressor' in args:
-            raise NotImplementedError("gencomm_b200: the NaiveCompressor is a training-only add-on (…_stage1.py:152-158)")
-        self.eval()
 
     @staticmethod
     def _make_message_extractor(args):
         return MessageExtractorv2(args['message_extractor']['in_ch'], args['message_extractor']['out_ch'])
-
-    def invalidate(self):
-        """Drop every packed-weight cache of the detector (after in-place parameter writes through ``p.data``)."""
-        for m in self.modules():
-            if m is not self and hasattr(m, "invalidate"):
-                m.invalidate()
-        for key in ("_heads", "_heads_single"):
-            h = getattr(self, key, None)
-            if h is not None:
-                h.invalidate()
-
-    def _load_from_state_dict(self, *args, **kwargs):
-        for key in ("_heads", "_heads_single"):      # the fused-heads helper is not a registered sub-module
-            h = getattr(self, key, None)
-            if h is not None:
-                h.invalidate()
-        return super()._load_from_state_dict(*args, **kwargs)
-
-    def set_encoder(self, modality_name, module):
-        """Plug in an encoder for a modality (e.g. the reference's own ``LiftSplatShoot`` instance): it is called as
-        ``module(data_dict, modality_name)`` like heter_encoders' classes and must return the BEV feature on the device."""
-        setattr(self, f"encoder_{modality_name}", module)
 
     # hooks the stage-2 class overrides
     def _before_gencomm(self, feature):
@@ -180,69 +77,21 @@ class HeterModelBaselineWGenComm(_HeadsMixin, nn.Module):
         affine_matrix = normalize_pairwise_tfm(data_dict['pairwise_t_matrix'], self.H, self.W, self.fake_voxel_size)
         record_len = data_dict['record_len']
 
-        counts = Counter(agent_modality_list)
+        # predraw: sampler noise of this frame on a side stream, issued between the encoder and the backbone: its generator
+        # kernels (HBM writes + ALU) run under the tensor-bound backbone instead of in front of the sampler (after the
+        # HBM-bound front end, not beside it; issued after the backbone instead, under the shrink header, it was measured
+        # 0.4 % slower: profiles/r02bk)
         features, messages = {}, {}
-        for m in self.modality_name_list:
-            if m not in counts:
-                continue
-            inp = data_dict[f'inputs_{m}']
-            if 'points' not in inp and 'batch_size' not in inp:
-                # the agent count is known on the host: spares PointPillarScatter's `.item()` sync (point_pillar_scatter.py:45)
-                data_dict = dict(data_dict)
-                data_dict[f'inputs_{m}'] = dict(inp, batch_size=counts[m])
-            encoder, backbone = getattr(self, f"encoder_{m}"), getattr(self, f"backbone_{m}")
-            shrinker = getattr(self, f"shrinker_{m}")
-            # raw points straight into this package's backbone: the canvas is written as its operand planes
-            planes_in = isinstance(encoder, PointPillar) and isinstance(backbone, BaseBEVBackbone) and 'points' in inp
-            try:
-                if planes_in:
-                    encoder.emit_planes = True
-                feature = encoder(data_dict, m)
-            finally:
-                if planes_in:
-                    encoder.emit_planes = False
-            if predraw:
-                # sampler noise of this frame on a side stream: its generator kernels (HBM writes + ALU) run under the
-                # tensor-bound backbone instead of in front of the sampler (after the HBM-bound front end, not beside it;
-                # issued after the backbone instead, under the shrink header, it was measured 0.4 % slower: profiles/r02bk)
-                self.gencomm.predraw()
-            if not isinstance(backbone, nn.Identity):
-                # the shrink header follows directly: the deblocks write its operand planes, no NCHW fp32 round trip
-                fused = isinstance(backbone, BaseBEVBackbone) and isinstance(shrinker, DownsampleConv)
-                try:
-                    if fused:
-                        backbone.emit_planes = True
-                    feature = backbone({"spatial_features": feature})['spatial_features_2d']
-                finally:
-                    if fused:
-                        backbone.emit_planes = False
-            feature = shrinker(feature)
+        for m, feature in self._encode(data_dict, self.gencomm.predraw if predraw else None):
             features[m] = feature
             messages[m] = getattr(self, f"message_extractor_{m}")(feature)
 
-        # camera feature maps cover the camera grid only: zero-pad them to the LiDAR extent (…_stage1.py:199-213)
         for m in features:
-            if self.sensor_type_dict[m] == "camera":
-                h, w = features[m].shape[-2:]
-                th, tw = int(h * getattr(self, f"crop_ratio_H_{m}")), int(w * getattr(self, f"crop_ratio_W_{m}"))
-                features[m] = center_crop(features[m], th, tw)
-                if self.CROP_MESSAGE:
-                    messages[m] = center_crop(messages[m], th, tw)
-
-        # restore the per-agent order from the per-modality batches (…_stage1.py:215-228)
-        if len(features) == 1 and all(a == agent_modality_list[0] for a in agent_modality_list):
-            m = agent_modality_list[0]
-            heter_feature_2d, heter_message = features[m], messages[m]
-            if heter_feature_2d.shape[0] != len(agent_modality_list):
-                raise ValueError("agent_modality_list does not match the number of encoded agents")
-        else:
-            seen = {m: 0 for m in self.modality_name_list}
-            f_list, m_list = [], []
-            for m in agent_modality_list:
-                f_list.append(features[m][seen[m]])
-                m_list.append(messages[m][seen[m]])
-                seen[m] += 1
-            heter_feature_2d, heter_message = torch.stack(f_list), torch.stack(m_list)
+            features[m] = self._pad_to_lidar(m, features[m])
+            if self.CROP_MESSAGE:
+                messages[m] = self._pad_to_lidar(m, messages[m])
+        heter_feature_2d = self._per_agent(features, agent_modality_list)
+        heter_message = self._per_agent(messages, agent_modality_list)
 
         if self.missing_message:   # robustness experiment: drop message cells of the non-ego agents (…_stage1.py:230-235)
             heter_message = heter_message.clone()
@@ -250,9 +99,7 @@ class HeterModelBaselineWGenComm(_HeadsMixin, nn.Module):
                 heter_message[i] *= torch.rand(heter_message.shape[1:], device=heter_message.device) > self.MISSING_KEEP
         conditions = heter_message
 
-        if self.supervise_single:
-            c, r, d = self._run_heads(heter_feature_2d, "_single")
-            output_dict.update({'cls_preds_single': c, 'reg_preds_single': r, 'dir_preds_single': d})
+        output_dict.update(self._single_preds(heter_feature_2d))
 
         gt_feature = heter_feature_2d
         state = self._before_gencomm(heter_feature_2d)
@@ -265,11 +112,6 @@ class HeterModelBaselineWGenComm(_HeadsMixin, nn.Module):
             heter_feature_2d = heter_feature_2d.unsqueeze(0)
         if hasattr(self, 'enhancer'):
             heter_feature_2d = self.enhancer(heter_feature_2d, affine_matrix, record_len)
-        fused_feature = self.fusion_net(heter_feature_2d, record_len, affine_matrix)
-        if self.shrink_flag:
-            fused_feature = self.shrink_conv(fused_feature)
-
-        cls_preds, reg_preds, dir_preds = self._run_heads(fused_feature)
-        output_dict.update({'cls_preds': cls_preds, 'reg_preds': reg_preds, 'dir_preds': dir_preds,
-                            'message': conditions})
+        output_dict.update(self._detect(heter_feature_2d, record_len, affine_matrix))
+        output_dict['message'] = conditions
         return output_dict

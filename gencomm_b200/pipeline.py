@@ -120,19 +120,26 @@ class DetectorPipeline:
         heads -> decode + rotated NMS -> boxes [F,1000,8,3], scores [F,1000], counts [F]
 
     ``shape``: "opv2v_h" (m1_att.yaml: C=128 at 64x128) or "v2xreal" (C=256, z +-15 m; synth.gencomm_v2xreal_args).
+    ``detector="baseline"``: ``HeterModelBaseline`` on the same arguments without the GenComm blocks -- the agents share
+    their full BEV features and the message extractor, sampler and Enhancer do not run (``precision`` must stay None).
     Everything is asynchronous on the current stream; weights are the seeded synthetic fill of synth.fill_state_dict."""
 
     def __init__(self, n_frames, n_agents, points_per_agent, shape="opv2v_h", fusion="att", device="cuda", seed=11,
-                 score_threshold=0.6, precision=None):
+                 score_threshold=0.6, precision=None, detector="gencomm"):
         from . import synth
+        from .heter_model_baseline import HeterModelBaseline
         from .heter_model_baseline_w_gencomm_stage1 import HeterModelBaselineWGenComm
         from .postprocess import VoxelPostprocessor
+        if detector not in ("gencomm", "baseline"):
+            raise ValueError(f"DetectorPipeline: detector {detector!r} -- 'gencomm' or 'baseline'")
         self.F, self.N, self.P = int(n_frames), int(n_agents), int(points_per_agent)
         self.device = torch.device(device)
         self.shape = shape
         self.args = synth.gencomm_v2xreal_args(fusion) if shape == "v2xreal" else synth.gencomm_stage1_args(fusion)
+        if detector == "baseline":
+            self.args = synth.without_gencomm(self.args)
         self.lidar_range = list(self.args["lidar_range"])
-        m = HeterModelBaselineWGenComm(self.args)
+        m = (HeterModelBaseline if detector == "baseline" else HeterModelBaselineWGenComm)(self.args)
         m.load_state_dict(synth.fill_state_dict(m.state_dict(), seed))
         self.model = m.to(self.device).eval()
         if precision is not None:
@@ -173,7 +180,7 @@ class DetectorPipeline:
         }
 
     def enable_stage_timing(self):
-        """Forward hooks that record CUDA events around every sub-module (current stream)."""
+        """Forward hooks that record CUDA events around every sub-module the detector has (current stream)."""
         self._marks = []
 
         def ev():
@@ -181,7 +188,9 @@ class DetectorPipeline:
             e.record()
             return e
         for name, label in DETECTOR_STAGES.items():
-            mod = getattr(self.model, name)
+            mod = getattr(self.model, name, None)
+            if mod is None:
+                continue
             mod.register_forward_pre_hook(lambda _m, _i, label=label: self._mark(label, 0))
             mod.register_forward_hook(lambda _m, _i, _o, label=label: self._mark(label, 1))
         self._ev = ev

@@ -216,6 +216,23 @@ def gencomm_stage2_hetero_args(fusion="att"):
     return a
 
 
+def without_gencomm(args):
+    """``model.args`` of a GenComm detector minus its GenComm blocks (sampler, Enhancer, message extractor): the arguments
+    of ``HeterModelBaseline``, the same detector sending full BEV features."""
+    return {k: v for k, v in args.items() if k not in ("gencomm", "diffcomm", "enhancer", "message_extractor")}
+
+
+def heter_baseline_args(fusion="att"):
+    """``HeterModelBaseline`` arguments of the LiDAR PointPillars agents of ``gencomm_stage1_args`` (OPV2V-H range, C=128
+    at 64x128) -- BASELINE.json configs 1-2."""
+    return without_gencomm(gencomm_stage1_args(fusion))
+
+
+def heter_baseline_hetero_args(fusion="att"):
+    """``HeterModelBaseline`` arguments of the LiDAR (m1) + camera (m2) agents of ``gencomm_stage2_hetero_args``."""
+    return without_gencomm(gencomm_stage2_hetero_args(fusion))
+
+
 def heter_frames(seed, record_len, n_points=30_000, max_cav=5):
     """Host inputs of a batch of collaborative frames for the full detector: per-agent clouds (list of [P,4] f32) and
     ``pairwise_t_matrix`` [B,L,L,4,4] f64; agents stay within ~40 m so their canvases overlap after the warp."""
